@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # CUDA arm (this repo)
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm (the reference's algorithm on host cores)
+    python bench.py --steps K --dump-outputs DIR             # + the last timed step's outputs as DIR/*.npy
 
 Workload (BASELINE.json configs[2], the one the metric's "1/2/4/8 B200" sharding
 is defined on): a channelizer batch of independent 2.4 MS/s complex-f32
@@ -37,6 +38,9 @@ OUT_CHUNK = 2048
 BYTES_PER_SAMPLE = 8.0 * (1.0 + OUT_RATE / SAMPLE_RATE)  # SURVEY.md 8(d): read once + written once
 METRIC = "complex MS/s via FreqShift->Filter->Downsampler"
 UNIT = "MS/s"
+# --dump-outputs writes at most this many bytes: a seeded sample of the streams when one step's output is larger
+# (4096 streams x 4096 complex64 samples = 128 MB at the default size)
+DUMP_BYTES = 32 << 20
 
 
 
@@ -272,6 +276,20 @@ def _time_pushes(torch, chain, sr, n, chunks, x_ptr, in_stride, y_ptr, cap, step
     return e0.elapsed_time(e1) / steps
 
 
+def dump_outputs(out_dir, torch, y, count):
+    """Writes what the last timed push returned to its caller, y[s, :count] per stream (complex64 as float32 pairs), for
+    a fixed, seeded sample of the streams that keeps the files within DUMP_BYTES: out_dir/output.npy [streams, count, 2]
+    float32, and the sampled stream indices as out_dir/output_streams.npy (float64)."""
+    S = y.shape[0]
+    k = min(S, max(1, DUMP_BYTES // max(8 * count, 1)))
+    n = min(count, DUMP_BYTES // (8 * k))
+    ids = np.sort(np.random.default_rng(20260000).choice(S, size=k, replace=False))
+    sample = y[torch.from_numpy(ids).to(y.device), :n].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "output.npy"), sample)
+    np.save(os.path.join(out_dir, "output_streams.npy"), ids.astype(np.float64))
+
+
 def _spot_check(rr, ctx, stages, ostages, flt, sr, n, chunks, x_host):
     """relative L2 error of the CUDA chain against the oracle on one small host-side stream (the parity spot check that
     goes with every configuration's throughput figure)"""
@@ -454,6 +472,8 @@ def run_cuda(args):
     k_all = chain.kernel_breakdown()
     chain.set_timing(False)
     plan = chain.plan
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, y, cnt)  # before anything else writes y
     if dist is not None:
         t = torch.tensor([elapsed_ms], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -751,7 +771,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the push-size sweep, the sustained run and the other configs")
     ap.add_argument("--traffic", type=float, default=None, help="dram bytes per launch from an ncu --set full capture")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0, a seeded sample of its streams) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm")
     if args.warmup < 3 and args.impl == "cuda":
         args.warmup = 3
     if args.impl == "reference":
