@@ -199,28 +199,36 @@ def test_front_runs_are_bit_reproducible(ctx):
 
 def test_front_full_baseline_size_on_device(ctx):
     """BASELINE.json config C3 at its full single-GPU size -- 4096 streams x 50 chunks x 4096 samples per push,
-    device resident (6.7 GB of input) -- through properties that need no oracle run at that size:
-    streams s and s + 2048 get identical samples and shifts and must come out bit-identical (independence,
-    determinism, no cross-stream leakage in the persistent kernels), three pushes, and three streams are checked
-    against the oracle sample by sample."""
+    device resident (6.7 GB of input), three pushes of the same samples -- with every stream checked.  The chain is
+    linear for a fixed shift: stream s is a_s*A + b_s*B (seeded weights of order 1) with shift class s mod 7 (7 is
+    coprime to the SM count, so the stream a persistent CTA runs just before s has another shift and other weights),
+    and must come out as a_s*ref(A, k) + b_s*ref(B, k) with the f64 oracle's ref: per stream, rel-L2 <= 3e-6 and
+    max |err| / rms <= 3e-5 (tests/test_gpu_layout.py explains the bounds)."""
+    import math
+
     import torch
 
     import radiorust_b200 as rr
 
-    sr, n, S, C = 2_400_000.0, 4096, 4096, 50
-    half = S // 2
+    sr, n, S, C, K = 2_400_000.0, 4096, 4096, 50, 7
     length = C * n
-    gen = torch.Generator(device="cuda")
-    gen.manual_seed(20260000 + 3 * 100000)
-    x = torch.empty((S, length, 2), device="cuda", dtype=torch.float32)
-    x[:half] = torch.randn((half, length, 2), device="cuda", dtype=torch.float32, generator=gen)
-    x[half:] = x[:half]
-    shifts = [float((s % half) * 577 % 2_400_000 - 1_200_000) for s in range(S)]   # SURVEY.md 8(d)
+    assert math.gcd(torch.cuda.get_device_properties(0).multi_processor_count, K) == 1
+    A = orc.synth_noise(20260000 + 3 * 100000, length, "f64")
+    B = orc.synth_noise(20260000 + 3 * 100000 + 1, length, "f64")
+    rng = np.random.default_rng(20260000 + 3 * 100000 + 2)
+    wa, wb = (0.5 + rng.random((2, S))) * np.exp(2j * np.pi * rng.random((2, S)))
+    A_d, B_d, a_d, b_d = (torch.from_numpy(v).cuda() for v in (A, B, wa, wb))
+    x = torch.empty((S, length), device="cuda", dtype=torch.complex64)
+    for s0 in range(0, S, 128):
+        x[s0:s0 + 128] = (a_d[s0:s0 + 128, None] * A_d[None] + b_d[s0:s0 + 128, None] * B_d[None]).to(torch.complex64)
+    del A_d, B_d
+    class_shift = [float((k * 577 * 293) % 2_400_000 - 1_200_000) for k in range(K)]   # SURVEY.md 8(d) style
     chain = rr.Chain(ctx, [rr.FreqShifter(0.0), rr.Filter.new(orc.lowpass(3000.0)), rr.Downsampler(2048, 48000.0, 6000.0)],
                      "f32", n_streams=S)
-    chain.set_shifts(0, shifts)
+    chain.set_shifts(0, [class_shift[s % K] for s in range(S)])
     cap = chain.max_output(sr, n, C + 1) + 2048
-    y = torch.zeros((S, cap, 2), device="cuda", dtype=torch.float32)
+    y = torch.zeros((S, cap), device="cuda", dtype=torch.complex64)
+    torch.cuda.synchronize()
     outs = []
     for push in range(3):
         cnt, rate = chain.push_device(sr, n, C, x.data_ptr(), length, y.data_ptr(), cap, cap)
@@ -229,21 +237,27 @@ def test_front_full_baseline_size_on_device(ctx):
         assert rate == 48000.0 and cnt > 0 and cnt % 2048 == 0
         # push 0: start-up chunks + k_front + k_poly2; push 1 (steady state): k_fused
         assert ("front+poly2" if push == 0 else "fused[") in chain.plan, chain.plan
-        got = y[:, :cnt].clone()
-        assert torch.equal(got[:half], got[half:])
-        assert bool(torch.isfinite(got).all())
-        outs.append(got)
+        outs.append(y[:, :cnt].cpu().numpy())
     chain.close()
-    for s in (0, 1000, 2047):
-        xs = x[s].cpu().numpy().view(np.complex64).reshape(-1)
-        oc = orc.Chain([orc.FreqShifter("f32", 1.0, shifts[s]), orc.Filter.new("f32", orc.lowpass(3000.0)),
-                        orc.Downsampler("f32", 2048, 48000.0, 6000.0)])
-        want = oc.run(sr, np.concatenate([xs, xs, xs]), n)
-        g = torch.cat([outs[0][s], outs[1][s], outs[2][s]]).cpu().numpy().view(np.complex64).reshape(-1)
-        assert g.shape == want.shape
-        assert orc.rel_l2(g, want) <= TOL
     del x, y
     torch.cuda.empty_cache()
+    got = np.concatenate(outs, axis=1)
+    ref = []
+    for base in (A, B):
+        ref.append(np.stack([orc.Chain([orc.FreqShifter("f64", 1.0, class_shift[k]), orc.Filter.new("f64", orc.lowpass(3000.0)),
+                                        orc.Downsampler("f64", 2048, 48000.0, 6000.0)]).run(sr, np.concatenate([base, base, base]), n)
+                             for k in range(K)]))
+    assert got.shape == (S, ref[0].shape[1]), (got.shape, ref[0].shape)
+    M = got.shape[1]
+    for s0 in range(0, S, 512):
+        cls = np.arange(s0, s0 + 512) % K
+        want = wa[s0:s0 + 512, None] * ref[0][cls] + wb[s0:s0 + 512, None] * ref[1][cls]
+        err = got[s0:s0 + 512].astype(np.complex128) - want
+        den = np.linalg.norm(want, axis=1)
+        rel = np.linalg.norm(err, axis=1) / den
+        mx = np.abs(err).max(axis=1) / (den / math.sqrt(M))
+        bad = np.flatnonzero(~((rel <= 3e-6) & (mx <= 3e-5)))
+        assert bad.size == 0, (s0 + bad[:8], rel[bad[:8]], mx[bad[:8]])
 
 
 def test_chain_destroy_releases_device_memory(ctx):
