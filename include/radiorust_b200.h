@@ -36,7 +36,7 @@ extern "C" {
 #endif
 
 #define RR_VERSION_MAJOR 0
-#define RR_VERSION_MINOR 4
+#define RR_VERSION_MINOR 5
 
 typedef struct rr_ctx rr_ctx;
 typedef struct rr_chain rr_chain;
@@ -264,6 +264,16 @@ int rr_chain_push(rr_chain* chain, double sample_rate, size_t chunk_len, size_t 
 int rr_chain_push_device(rr_chain* chain, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in,
                          size_t in_stride, void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count,
                          double* out_sample_rate);
+/* Every stream reads the same n_chunks*chunk_len input samples (one row): a channelizer tuning all its streams
+ * out of one wideband input.  Stream state (NCO phase, Filter history, resampler rings, ...) stays per stream;
+ * outputs are laid out as for rr_chain_push[_device].  The results equal a push of the row replicated into
+ * every stream, bit for bit, whenever both take the same plan.  The host form copies the row once (len samples,
+ * not n_streams*len); the device form reads it in place, so its input costs no memory per stream.  Contract,
+ * refusals and failure handling as for the per-stream pushes; the two kinds may be mixed on one chain. */
+int rr_chain_push_shared(rr_chain* chain, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in,
+                         void* host_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate);
+int rr_chain_push_shared_device(rr_chain* chain, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in,
+                                void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate);
 int rr_chain_sync(rr_chain* chain);
 /* Copy `n_samples` samples per stream from one device buffer to another (a buffer of another GPU opened with rr_ipc_open,
  * for example) on the chain's copy stream -- a copy engine, no SM -- behind everything queued on the chain so far: a

@@ -396,6 +396,52 @@ class Chain:
         )
         return cnt.value, rate.value
 
+    def push_shared(self, sample_rate: float, x: np.ndarray, chunk_len: int, out: Optional[np.ndarray] = None):
+        """Push one 1-D row ``x`` from HOST memory into every stream (``rr_chain_push_shared``): a channelizer tuning all
+        its streams out of one wideband input.  Returns ``(y, out_rate)`` with ``y`` of shape ``[n_streams, out_count]``."""
+        x = np.asarray(x)
+        assert x.ndim == 1, "one row, read by every stream"
+        assert x.dtype == self.cdtype and x.strides[0] == x.itemsize
+        total = x.shape[0]
+        assert total % chunk_len == 0
+        n_chunks = total // chunk_len if chunk_len else 0
+        cap = self.max_output(sample_rate, chunk_len, n_chunks)
+        if out is None:
+            out = np.empty((self.n_streams, max(cap, 1)), dtype=self.cdtype)
+        cnt = C.c_size_t()
+        rate = C.c_double()
+        check(
+            self._lib.rr_chain_push_shared(
+                self._h, float(sample_rate), chunk_len, n_chunks, x.ctypes.data, out.ctypes.data, out.shape[1],
+                out.strides[0] // out.itemsize, C.byref(cnt), C.byref(rate),
+            )
+        )
+        self.sync()
+        return out[:, : cnt.value], rate.value
+
+    def push_shared_device(self, sample_rate, chunk_len, n_chunks, dev_in: int, dev_out: int, out_capacity: int, out_stride: int):
+        """``rr_chain_push_shared_device``: every stream reads the row at ``dev_in`` (raw device pointers); returns
+        ``(out_count, out_rate)``; asynchronous."""
+        cnt = C.c_size_t()
+        rate = C.c_double()
+        check(
+            self._lib.rr_chain_push_shared_device(
+                self._h, float(sample_rate), chunk_len, n_chunks, dev_in, dev_out, out_capacity, out_stride, C.byref(cnt), C.byref(rate),
+            )
+        )
+        return cnt.value, rate.value
+
+    def push_shared_host_async(self, sample_rate, chunk_len, n_chunks, host_in: int, host_out: int, out_capacity: int, out_stride: int):
+        """``rr_chain_push_shared`` with raw (pinned) host pointers; asynchronous until :meth:`sync`."""
+        cnt = C.c_size_t()
+        rate = C.c_double()
+        check(
+            self._lib.rr_chain_push_shared(
+                self._h, float(sample_rate), chunk_len, n_chunks, host_in, host_out, out_capacity, out_stride, C.byref(cnt), C.byref(rate),
+            )
+        )
+        return cnt.value, rate.value
+
     def copy_out_async(self, dst_dev: int, dst_stride: int, src_dev: int, src_stride: int, n_samples: int):
         """``rr_chain_copy_out_async``: copy-engine copy of a push's outputs (raw device pointers), behind the queued work."""
         check(self._lib.rr_chain_copy_out_async(self._h, dst_dev, dst_stride, src_dev, src_stride, n_samples))

@@ -866,6 +866,7 @@ struct FilterIo {
     long long in_stride = 0;
     size_t n = 0, n_chunks = 0;
     Stage* nco = nullptr;
+    bool shared = false;  // `in` is the row of a shared push that every stream reads (in_stride 0, S > 1)
 };
 
 // run the stand-alone NCO kernel over chunks [c0, c0+k) into the NCO stage's buffer
@@ -1403,7 +1404,7 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
             const long long I_hi = m_hi / Qq;
             bool done = false;
             if constexpr (std::is_same<T, float>::value) {
-                const bool tma_ok = ((uintptr_t)a.in % 16 == 0) && (S == 1 || a.in_stride % 2 == 0) && a.len < (1LL << 31);
+                const bool tma_ok = ((uintptr_t)a.in % 16 == 0) && (S == 1 || io.shared || a.in_stride % 2 == 0) && a.len < (1LL << 31);
                 // ---- k_fused: front end + low-rate part in one persistent kernel (u stays in shared memory).  Steady
                 // state only: the whole push is polyphase, the previous push left its last Lmax rows of u behind, and
                 // there are enough streams to give every SM whole streams; everything else takes k_front + k_poly2.
@@ -1459,7 +1460,7 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
                         f.hist_fused_jlo = cover_hi - hfrom;
                         f.hist_fused_jfirst = hstart - hfrom;
                     }
-                    RR_TIMED_LAUNCH(c, "k_fused", 1, rr::launch_fused(S, fu, c->ctx->sm_count, st));
+                    RR_TIMED_LAUNCH(c, "k_fused", 1, rr::launch_fused(S, fu, io.shared, c->ctx->sm_count, st));
                     ds.ucache_valid = true;
                     ds.ucache_rows = n_out + Lh;
                     ds.ucache_ptr = kb.p;
@@ -1536,7 +1537,7 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
                             f.hist_fused_jlo = cover_hi - hfrom;
                             f.hist_fused_jfirst = hstart - hfrom;
                         }
-                        RR_TIMED_LAUNCH(c, "k_front", 1, rr::launch_front(RK, S, fa, st));
+                        RR_TIMED_LAUNCH(c, "k_front", 1, rr::launch_front(RK, S, fa, io.shared, st));
                         rr::PolyArgs<float> b{};
                         b.in = ub.p;
                         b.in_stride = u_stride;
@@ -1600,7 +1601,7 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
                             b.out_stride *= sab_run;
                             b.out2_stride *= sab_run;
                         }
-                        RR_TIMED_LAUNCH(c, "k_poly2", 1, rr::launch_poly2(G2, S2, b, st));
+                        RR_TIMED_LAUNCH(c, "k_poly2", 1, rr::launch_poly2(G2, S2, b, false, st));
                         ds.ucache_valid = true;
                         ds.ucache_rows = n_rows;
                         // the last Lmax rows of [history rows | new rows] of this push
@@ -1656,7 +1657,7 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
                             f.hist_fused_jfirst = hstart - hfrom;
                         }
                         if (ds.frontq_wide) RR_TIMED_LAUNCH(c, "k_front_wide", 1, rr::launch_front_wide(RQ, S, fa, st));
-                        else RR_TIMED_LAUNCH(c, "k_front", 1, rr::launch_front(RQ, S, fa, st));
+                        else RR_TIMED_LAUNCH(c, "k_front", 1, rr::launch_front(RQ, S, fa, io.shared, st));
                         rr::PolyArgs<float> b{};
                         b.in = ub.p;
                         b.in_stride = u_stride;
@@ -1714,7 +1715,7 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
                     a.out = obase;
                     a.out_stride = ostride;
                     a.hist2 = f.hist2[f.hist_cur].p;
-                    RR_TIMED_LAUNCH(c, "k_poly2", 1, rr::launch_poly2(G2, S, a, st));
+                    RR_TIMED_LAUNCH(c, "k_poly2", 1, rr::launch_poly2(G2, S, a, io.shared, st));
                     done = true;
                     used_poly2 = true;
                 }
@@ -1741,9 +1742,11 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
     return RR_OK;
 }
 
+// shared: every stream reads the row at dev_in (in_stride is 0).  The stride travels with the input view, so every
+// stage that reads the push's input sees it; the TMA launchers take their shared-row form on a zero stride.
 template <typename T>
-int run_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride, void* dev_out,
-             size_t out_capacity, size_t out_stride, size_t* out_count, double* out_rate) {
+int run_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride, bool shared,
+             void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_rate) {
     const int S = c->S;
     const int ns = (int)c->st.size();
     cudaStream_t st = c->stream;
@@ -1751,7 +1754,8 @@ int run_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks,
     in.chunk_len = chunk_len;
     in.n_chunks = n_chunks;
     in.rate = sample_rate;
-    if (chunk_len * n_chunks > in_stride && S > 1) return fail(RR_ERR_INVALID, "in_stride smaller than the pushed samples");
+    if (shared) in_stride = 0;
+    else if (chunk_len * n_chunks > in_stride && S > 1) return fail(RR_ERR_INVALID, "in_stride smaller than the pushed samples");
 
     // ---- dry run: output shape + capacity before anything is touched -------
     {
@@ -1964,6 +1968,7 @@ int run_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks,
                 }
                 FilterIo io;
                 io.in = cur.p;
+                io.shared = shared && S > 1 && cur.p == dev_in;  // still the pushed row (a Rechunker view keeps it)
                 io.in_stride = cur.stride;
                 io.n = n;
                 io.n_chunks = cur.sh.n_chunks;
@@ -2713,22 +2718,27 @@ size_t rr_chain_max_output(rr_chain* c, double sample_rate, size_t chunk_len, si
     return out.len();
 }
 
-int rr_chain_push_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride,
-                         void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
+}  // extern "C"
+
+namespace {
+
+// rr_chain_push_device / rr_chain_push_shared_device (shared: one input row for every stream, in_stride ignored)
+int push_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride, bool shared,
+                void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
     if (!c) return fail(RR_ERR_INVALID, "null chain");
     if (out_count) *out_count = 0;
     if (n_chunks == 0 || chunk_len == 0) return RR_OK;
-    if (!dev_in) return fail(RR_ERR_INVALID, "rr_chain_push_device: dev_in is null");
+    if (!dev_in) return fail(RR_ERR_INVALID, shared ? "rr_chain_push_shared_device: dev_in is null" : "rr_chain_push_device: dev_in is null");
     if (chunk_len > (size_t)1 << 30 || n_chunks > (size_t)1 << 30) return fail(RR_ERR_INVALID, "push too large");
     RR_CUDA(cudaSetDevice(c->ctx->device));
     (void)cudaGetLastError();  // a stale error of an unrelated earlier call (another library in the process) is not ours
     c->push_mutated = false;
     int r;
     if (c->dtype == RR_C32)
-        r = run_push<float>(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, dev_out, out_capacity, out_stride, out_count,
+        r = run_push<float>(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, shared, dev_out, out_capacity, out_stride, out_count,
                             out_sample_rate);
     else
-        r = run_push<double>(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, dev_out, out_capacity, out_stride, out_count,
+        r = run_push<double>(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, shared, dev_out, out_capacity, out_stride, out_count,
                              out_sample_rate);
     if (r != RR_OK && c->push_mutated) {
         // A failure behind the dry run (allocation, CUDA error) left some stages advanced and others not.  The stream
@@ -2743,16 +2753,17 @@ int rr_chain_push_device(rr_chain* c, double sample_rate, size_t chunk_len, size
     return r;
 }
 
-int rr_chain_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in, size_t in_stride,
-                  void* host_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
+// rr_chain_push / rr_chain_push_shared (shared: one input row of len samples is staged and read by every stream)
+int push_host(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in, size_t in_stride, bool shared,
+              void* host_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
     if (!c) return fail(RR_ERR_INVALID, "null chain");
     if (out_count) *out_count = 0;
     if (n_chunks == 0 || chunk_len == 0) return RR_OK;
-    if (!host_in) return fail(RR_ERR_INVALID, "rr_chain_push: host_in is null");
+    if (!host_in) return fail(RR_ERR_INVALID, shared ? "rr_chain_push_shared: host_in is null" : "rr_chain_push: host_in is null");
     RR_CUDA(cudaSetDevice(c->ctx->device));
     const size_t len = chunk_len * n_chunks;
     const size_t S = (size_t)c->S;
-    if (S > 1 && in_stride < len) return fail(RR_ERR_INVALID, "in_stride smaller than the pushed samples");
+    if (!shared && S > 1 && in_stride < len) return fail(RR_ERR_INVALID, "in_stride smaller than the pushed samples");
     // everything that can be refused is refused before anything is enqueued or any state advances
     Shape sh_in, sh_out;
     sh_in.chunk_len = chunk_len;
@@ -2775,12 +2786,13 @@ int rr_chain_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_ch
     const int b = c->slot;
     const size_t ocap = max_out ? max_out : 1;
     // (a staging buffer that has to grow is freed first: cudaFree waits for the work that still uses it)
-    RR_TRY(c->stage_in[b].ensure(S * len * c->esz));
+    const size_t in_rows = shared ? 1 : S;
+    RR_TRY(c->stage_in[b].ensure(in_rows * len * c->esz));
     RR_TRY(c->stage_out[b].ensure(S * ocap * c->esz));
     // H2D of this push: behind the kernels of the push before last, which read the same slot
     RR_CUDA(cudaStreamWaitEvent(c->h2d_stream, c->ev_comp[b], 0));
-    if (in_stride == len || S == 1)  // contiguous: one linear copy
-        RR_CUDA(cudaMemcpyAsync(c->stage_in[b].p, host_in, S * len * c->esz, cudaMemcpyHostToDevice, c->h2d_stream));
+    if (in_rows == 1 || in_stride == len)  // contiguous: one linear copy
+        RR_CUDA(cudaMemcpyAsync(c->stage_in[b].p, host_in, in_rows * len * c->esz, cudaMemcpyHostToDevice, c->h2d_stream));
     else
         RR_CUDA(cudaMemcpy2DAsync(c->stage_in[b].p, len * c->esz, host_in, in_stride * c->esz, len * c->esz, S, cudaMemcpyHostToDevice,
                                   c->h2d_stream));
@@ -2789,8 +2801,8 @@ int rr_chain_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_ch
     RR_CUDA(cudaStreamWaitEvent(c->stream, c->ev_h2d[b], 0));
     RR_CUDA(cudaStreamWaitEvent(c->stream, c->ev_d2h[b], 0));
     size_t produced = 0;
-    RR_TRY(rr_chain_push_device(c, sample_rate, chunk_len, n_chunks, c->stage_in[b].p, len, c->stage_out[b].p, max_out, ocap, &produced,
-                                out_sample_rate));
+    RR_TRY(push_device(c, sample_rate, chunk_len, n_chunks, c->stage_in[b].p, len, shared, c->stage_out[b].p, max_out, ocap, &produced,
+                       out_sample_rate));
     RR_CUDA(cudaEventRecord(c->ev_comp[b], c->stream));
     if (produced > 0) {
         RR_CUDA(cudaStreamWaitEvent(c->d2h_stream, c->ev_comp[b], 0));
@@ -2804,6 +2816,32 @@ int rr_chain_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_ch
     c->slot ^= 1;
     if (out_count) *out_count = produced;
     return RR_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rr_chain_push_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride,
+                         void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
+    return push_device(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, false, dev_out, out_capacity, out_stride, out_count,
+                       out_sample_rate);
+}
+
+int rr_chain_push_shared_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, void* dev_out,
+                                size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
+    return push_device(c, sample_rate, chunk_len, n_chunks, dev_in, 0, true, dev_out, out_capacity, out_stride, out_count, out_sample_rate);
+}
+
+int rr_chain_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in, size_t in_stride,
+                  void* host_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
+    return push_host(c, sample_rate, chunk_len, n_chunks, host_in, in_stride, false, host_out, out_capacity, out_stride, out_count,
+                     out_sample_rate);
+}
+
+int rr_chain_push_shared(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in, void* host_out,
+                         size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
+    return push_host(c, sample_rate, chunk_len, n_chunks, host_in, 0, true, host_out, out_capacity, out_stride, out_count, out_sample_rate);
 }
 
 // Device-to-device copy of `n_samples` samples per stream on the chain's copy stream (copy engine, no SM), ordered

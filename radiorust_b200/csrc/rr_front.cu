@@ -55,7 +55,8 @@ __device__ __forceinline__ pc lds_front(uint32_t addr) {
     return r;
 }
 
-template <int RK, bool HAS_NCO>
+// SHARED_IN: every stream reads the same input row (the input map holds that one row; the history map stays per stream)
+template <int RK, bool HAS_NCO, bool SHARED_IN>
 __global__ void __launch_bounds__(FR_WARPS * 32, 4) k_front(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_h, const FrontArgs a) {
     static_assert(RK == 10 || RK == 16, "results leave as 16-byte pairs: 6 + 4 per lane pair for ten columns, 8 + 8 for sixteen");
     constexpr int RK_SPLIT = RK == 10 ? 6 : RK / 2;  // lane hh = 0 stores results [0, RK_SPLIT), lane hh = 1 the rest
@@ -157,7 +158,7 @@ __global__ void __launch_bounds__(FR_WARPS * 32, 4) k_front(const __grid_constan
             asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(tile_bytes) : "memory");
             asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
                              tiles_s + (k % FR_STAGES) * tile_stride),
-                         "l"(from_in ? &tmap : &tmap_h), "r"(bar), "r"(from_in ? pos0 : pos0 + hist32), "r"(0), "r"(s)
+                         "l"(from_in ? &tmap : &tmap_h), "r"(bar), "r"(from_in ? pos0 : pos0 + hist32), "r"(0), "r"(SHARED_IN && from_in ? 0 : s)
                          : "memory");
         }
     };
@@ -405,7 +406,7 @@ bool front_supported(int rank_pad, long long P) {
     return (rank_pad == 10 || rank_pad == 16) && P >= 2 && P <= 254 && (P % 2) == 0 && front_encode_fn() != nullptr;
 }
 
-cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a0, cudaStream_t st) {
+cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a0, bool shared, cudaStream_t st) {
     EncodeFn enc = front_encode_fn();
     if (!enc || (rank_pad != 10 && rank_pad != 16)) return cudaErrorNotSupported;
     FrontArgs a = a0;
@@ -415,10 +416,12 @@ cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a0, cudaS
     int ctas = (tiles + FR_WARPS * 64 - 1) / (FR_WARPS * 64);
     while ((long long)n_streams * ctas < 592 && ctas * FR_WARPS < tiles) ++ctas;
     a.tiles_per_warp = (tiles + ctas * FR_WARPS - 1) / (ctas * FR_WARPS);
-    // the stream as overlapping rows of P samples: element (c0, i, s) = in[s*in_stride + c0 + i*P]
+    // the stream as overlapping rows of P samples: element (c0, i, s) = in[s*in_stride + c0 + i*P].  shared: one row
+    // that every stream reads, mapped once (a zero stride cannot be encoded)
+    if (shared != (n_streams > 1 && a.in_stride == 0)) return cudaErrorInvalidValue;
     CUtensorMap tm;
-    const cuuint64_t dims[3] = {(cuuint64_t)a.len, (cuuint64_t)FR_ROWS, (cuuint64_t)n_streams};
-    const cuuint64_t sstride = n_streams > 1 ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
+    const cuuint64_t dims[3] = {(cuuint64_t)a.len, (cuuint64_t)FR_ROWS, (cuuint64_t)(shared ? 1 : n_streams)};
+    const cuuint64_t sstride = n_streams > 1 && !shared ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
     const cuuint64_t strides[2] = {(cuuint64_t)a.P * 8, sstride};
     const int pitch = a.P + ((a.P & 3) == 0 ? 2 : 0);
     const cuuint32_t box[3] = {(cuuint32_t)pitch, (cuuint32_t)FR_ROWS, 1};
@@ -445,11 +448,21 @@ cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a0, cudaS
         if (e == cudaSuccess) kern<<<grid, FR_WARPS * 32, smem, st>>>(tm, tmh, a);
     };
     if (rank_pad == 10) {
-        if (a.nco) go(k_front<10, true>);
-        else go(k_front<10, false>);
+        if (shared) {
+            if (a.nco) go(k_front<10, true, true>);
+            else go(k_front<10, false, true>);
+        } else {
+            if (a.nco) go(k_front<10, true, false>);
+            else go(k_front<10, false, false>);
+        }
     } else {
-        if (a.nco) go(k_front<16, true>);
-        else go(k_front<16, false>);
+        if (shared) {
+            if (a.nco) go(k_front<16, true, true>);
+            else go(k_front<16, false, true>);
+        } else {
+            if (a.nco) go(k_front<16, true, false>);
+            else go(k_front<16, false, false>);
+        }
     }
     if (e != cudaSuccess) return e;
     return cudaGetLastError();

@@ -186,8 +186,9 @@ __device__ __forceinline__ void f_steps(pc (&acc)[FRK], const float4* __restrict
 }  // namespace
 
 // FW front-end warps, ring depth D per warp, NB parked spectra per inverse round; PT: decimation factor known at
-// compile time (the front end's step loop is unrolled completely) or 0 (any even P)
-template <int FW, int D, int NB, bool HAS_NCO, int PT>
+// compile time (the front end's step loop is unrolled completely) or 0 (any even P); SHARED_IN: every stream reads
+// the same input row (the tensor map holds that one row, the copies address stream 0)
+template <int FW, int D, int NB, bool HAS_NCO, int PT, bool SHARED_IN>
 __global__ void __launch_bounds__(T_THREADS + 32 * FW, 1)
 k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n_streams) {
     extern __shared__ __align__(128) unsigned char smem[];
@@ -291,7 +292,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
                     mb_expect_tx(rbar + i_slot * 8, (uint32_t)geo.slot_bytes);
                     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
                                      ring_s + i_slot * geo.slot_stride),
-                                 "l"(&tmap), "r"(rbar + i_slot * 8), "r"(pos0 + coff - sh * P), "r"(sh), "r"((int)blockIdx.x + so * (int)gridDim.x)
+                                 "l"(&tmap), "r"(rbar + i_slot * 8), "r"(pos0 + coff - sh * P), "r"(sh), "r"(SHARED_IN ? 0 : (int)blockIdx.x + so * (int)gridDim.x)
                                  : "memory");
                 }
                 i_slot = (i_slot + 1 == D) ? 0 : i_slot + 1;
@@ -786,7 +787,7 @@ template <int FW, int D, int NB> size_t fused_smem(int P, int Lmax) {
     return b;
 }
 
-template <int FW, int D, int NB>
+template <int FW, int D, int NB, bool SHARED_IN>
 cudaError_t launch_cfg(int n_streams, const FusedArgs& a, const CUtensorMap& tm, int sm_count, cudaStream_t st) {
     const size_t smem = fused_smem<FW, D, NB>(a.P, a.Lmax);
     if (smem > (size_t)227 * 1024) return cudaErrorInvalidConfiguration;
@@ -796,9 +797,9 @@ cudaError_t launch_cfg(int n_streams, const FusedArgs& a, const CUtensorMap& tm,
     // loads to go through the uniform datapath (with a run-time loop they are vector LDC loads and the kernel is slower
     // than k_front + k_poly2).  Common SDR ratios: 2.4 MS/s, 1.92 MS/s, 960 kS/s -> 48 kS/s.
     switch (a.P) {
-        case 50: kern = a.nco ? k_fused<FW, D, NB, true, 50> : k_fused<FW, D, NB, false, 50>; break;
-        case 40: kern = a.nco ? k_fused<FW, D, NB, true, 40> : k_fused<FW, D, NB, false, 40>; break;
-        case 20: kern = a.nco ? k_fused<FW, D, NB, true, 20> : k_fused<FW, D, NB, false, 20>; break;
+        case 50: kern = a.nco ? k_fused<FW, D, NB, true, 50, SHARED_IN> : k_fused<FW, D, NB, false, 50, SHARED_IN>; break;
+        case 40: kern = a.nco ? k_fused<FW, D, NB, true, 40, SHARED_IN> : k_fused<FW, D, NB, false, 40, SHARED_IN>; break;
+        case 20: kern = a.nco ? k_fused<FW, D, NB, true, 20, SHARED_IN> : k_fused<FW, D, NB, false, 20, SHARED_IN>; break;
         default: return cudaErrorNotSupported;
     }
     const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -840,7 +841,7 @@ cudaError_t fused_upload_coef(int slot, const float* acoef, int P, cudaStream_t 
     return cudaMemcpyToSymbolAsync(c_fcoef, acoef, n * sizeof(float), (size_t)slot * kFusedSlotFloats * sizeof(float), cudaMemcpyHostToDevice, st);
 }
 
-cudaError_t launch_fused(int n_streams, const FusedArgs& a0, int sm_count, cudaStream_t st) {
+cudaError_t launch_fused(int n_streams, const FusedArgs& a0, bool shared, int sm_count, cudaStream_t st) {
     EncodeFn enc = fused_encode_fn();
     if (!enc) return cudaErrorNotSupported;
     FusedArgs a = a0;
@@ -849,10 +850,12 @@ cudaError_t launch_fused(int n_streams, const FusedArgs& a0, int sm_count, cudaS
     if ((uintptr_t)a.ukeep_in % 16 != 0 || (n_streams > 1 && a.ukeep_in_stride % 2 != 0)) return cudaErrorInvalidValue;
     const FusedGeom geo = fused_geom(a.P);
     // the stream as overlapping rows of P samples: element (c0, i, s) = in[s*in_stride + c0 + i*P]; a box is half a
-    // row wide and F_ROWS rows tall
+    // row wide and F_ROWS rows tall.  shared: one row that every stream reads (a zero stride cannot be encoded; the map
+    // holds the row once and the kernel's shared form addresses it)
+    if (shared != (n_streams > 1 && a.in_stride == 0)) return cudaErrorInvalidValue;
     CUtensorMap tm;
-    const cuuint64_t dims[3] = {(cuuint64_t)a.len, (cuuint64_t)F_ROWS, (cuuint64_t)n_streams};
-    const cuuint64_t sstride = n_streams > 1 ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
+    const cuuint64_t dims[3] = {(cuuint64_t)a.len, (cuuint64_t)F_ROWS, (cuuint64_t)(shared ? 1 : n_streams)};
+    const cuuint64_t sstride = n_streams > 1 && !shared ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
     const cuuint64_t strides[2] = {(cuuint64_t)a.P * 8, sstride};
     const cuuint32_t box[3] = {(cuuint32_t)geo.hp, (cuuint32_t)F_ROWS, 1};
     const cuuint32_t estr[3] = {1, 1, 1};
@@ -866,9 +869,15 @@ cudaError_t launch_fused(int n_streams, const FusedArgs& a0, int sm_count, cudaS
         cfg = 0;
         if (const char* e = std::getenv("RR_FUSED_CFG")) cfg = std::atoi(e);
     }
+    if (shared) {
+        switch (cfg) {
+            case 1: return launch_cfg<6, 2, 8, true>(n_streams, a, tm, sm_count, st);
+            default: return launch_cfg<7, 2, 5, true>(n_streams, a, tm, sm_count, st);
+        }
+    }
     switch (cfg) {
-        case 1: return launch_cfg<6, 2, 8>(n_streams, a, tm, sm_count, st);
-        default: return launch_cfg<7, 2, 5>(n_streams, a, tm, sm_count, st);
+        case 1: return launch_cfg<6, 2, 8, false>(n_streams, a, tm, sm_count, st);
+        default: return launch_cfg<7, 2, 5, false>(n_streams, a, tm, sm_count, st);
     }
 }
 

@@ -217,7 +217,8 @@ int poly2_pick_G(long long P);
 size_t poly2_smem_bytes(int G, int nbpc);
 // position (complex elements) of bin k of branch p = r*G + g in the device table
 long long poly2_table_index(int G, int r, int g, int k);
-cudaError_t launch_poly2(int G, int n_streams, const PolyArgs<float>& a, cudaStream_t st);
+// shared_in: every stream reads the one row at a.in (a.in_stride == 0, n_streams > 1); a zero stride without it is refused
+cudaError_t launch_poly2(int G, int n_streams, const PolyArgs<float>& a, bool shared_in, cudaStream_t st);
 
 // ---- k_front (rr_front.cu): rank-reduced front end u_c[i] = sum_p a_c[p] * x'[i*P + p] (f32, Q == 1).
 // k_poly2 then runs on u as a stream of `rank_pad` branches.
@@ -249,7 +250,7 @@ struct FrontArgs {
     int kept_rows;
 };
 bool front_supported(int rank_pad, long long P);
-cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a, cudaStream_t st);
+cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a, bool shared_in, cudaStream_t st);  // shared_in: as launch_poly2
 // k_front_wide (rr_front_wide.cu): the same front end for any P (odd, thousands), 16 or 32 columns; `acoef` is
 // [P][rank_pad]; kept rows are not taken
 bool front_wide_supported(int rank_pad, long long P);
@@ -287,7 +288,7 @@ struct FusedArgs {
 bool fused_supported(int rank_pad, long long P, int Lmax);
 int fused_coef_slots();
 cudaError_t fused_upload_coef(int slot, const float* acoef, int P, cudaStream_t st);
-cudaError_t launch_fused(int n_streams, const FusedArgs& a, int sm_count, cudaStream_t st);
+cudaError_t launch_fused(int n_streams, const FusedArgs& a, bool shared_in, int sm_count, cudaStream_t st);  // shared_in: as launch_poly2
 
 // new hist2 = last 2n post-NCO samples of [hist2_in | in]; only entries [j_lo, j_hi) (j_hi < 0: 2n) -- the
 // others were written by k_front

@@ -170,7 +170,8 @@ __device__ __forceinline__ void pass1_store(pc (&v)[32], uint32_t tw_row, uint32
 // One CTA = two independent halves (own stream, shared memory, mbarriers, named barrier).
 // SINGLE: P <= G, one round per block (the low-rate part behind k_front): nothing is accumulated over
 // rounds, the products go straight to the warp's strip and the block needs one barrier.
-template <int G, bool HAS_NCO, bool SINGLE>
+// SHARED_IN: every stream reads the same input row (the tensor map holds that one row, the copies address stream 0)
+template <int G, bool HAS_NCO, bool SINGLE, bool SHARED_IN>
 __global__ void __launch_bounds__(2 * P2Cfg<G>::THREADS, 1) k_poly2(const __grid_constant__ CUtensorMap tmap, const PolyArgs<float> a, const int n_streams) {
     using C = P2Cfg<G>;
     constexpr int THREADS = C::THREADS, PITCH = C::PITCH;
@@ -243,7 +244,7 @@ __global__ void __launch_bounds__(2 * P2Cfg<G>::THREADS, 1) k_poly2(const __grid
                          "r"((uint32_t)C::TILE_BYTES), "r"(bar)
                          : "memory");
         } else {
-            tma_load_4d(dst, &tmap, bar, boff + (Rg % NR) * G, 0, 0, ss);
+            tma_load_4d(dst, &tmap, bar, boff + (Rg % NR) * G, 0, 0, SHARED_IN ? 0 : ss);
         }
     };
 
@@ -602,7 +603,7 @@ EncodeFn encode_fn() {
     return fn;
 }
 
-template <int G> cudaError_t launch_g(int n_streams, const PolyArgs<float>& a0, const CUtensorMap& tm, cudaStream_t st) {
+template <int G> cudaError_t launch_g(int n_streams, const PolyArgs<float>& a0, const CUtensorMap& tm, bool shared, cudaStream_t st) {
     using C = P2Cfg<G>;
     PolyArgs<float> a = a0;
     // EXPERIMENT (RR_P2_ONE_HALF_PER_SM=1): one half per CTA and one CTA per SM -- how fast is a lone half?
@@ -627,8 +628,14 @@ template <int G> cudaError_t launch_g(int n_streams, const PolyArgs<float>& a0, 
     const dim3 grid(gx, gy);
     void (*kern)(const CUtensorMap, const PolyArgs<float>, const int);
     const bool single = a.P <= G;
-    if (a.nco) kern = single ? k_poly2<G, true, true> : k_poly2<G, true, false>;
-    else kern = single ? k_poly2<G, false, true> : k_poly2<G, false, false>;
+    if (shared) {
+        if (a.nco) kern = single ? k_poly2<G, true, true, true> : k_poly2<G, true, false, true>;
+        else kern = single ? k_poly2<G, false, true, true> : k_poly2<G, false, false, true>;
+    } else if (a.nco) {
+        kern = single ? k_poly2<G, true, true, false> : k_poly2<G, true, false, false>;
+    } else {
+        kern = single ? k_poly2<G, false, true, false> : k_poly2<G, false, false, false>;
+    }
     const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kern<<<grid, halves * C::THREADS, smem, st>>>(tm, a, n_streams);
@@ -665,20 +672,23 @@ long long poly2_table_index(int G, int r, int g, int k) {
     return ((((long long)r * 2 + which) * 8 + (k2 >> 1)) * threads + tid) * 2 + (k2 & 1);
 }
 
-cudaError_t launch_poly2(int G, int n_streams, const PolyArgs<float>& a, cudaStream_t st) {
+cudaError_t launch_poly2(int G, int n_streams, const PolyArgs<float>& a, bool shared, cudaStream_t st) {
     EncodeFn enc = encode_fn();
     if (!enc) return cudaErrorNotSupported;
-    // the stream as overlapping rows: element (c0, i_lo, i_hi, s) = in[s*in_stride + c0 + (i_lo + 256*i_hi)*P]
+    // the stream as overlapping rows: element (c0, i_lo, i_hi, s) = in[s*in_stride + c0 + (i_lo + 256*i_hi)*P].
+    // shared: one row that every stream reads, mapped once (a zero stride cannot be encoded).  The low-rate part on u,
+    // streams-as-blocks form included, reads per-stream rows.
+    if (shared != (n_streams > 1 && a.in_stride == 0)) return cudaErrorInvalidValue;
     CUtensorMap tm;
-    const cuuint64_t dims[4] = {(cuuint64_t)a.len, (cuuint64_t)ROWS_BOX, (cuuint64_t)(K2 / ROWS_BOX), (cuuint64_t)n_streams};
-    const cuuint64_t sstride = n_streams > 1 ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
+    const cuuint64_t dims[4] = {(cuuint64_t)a.len, (cuuint64_t)ROWS_BOX, (cuuint64_t)(K2 / ROWS_BOX), (cuuint64_t)(shared ? 1 : n_streams)};
+    const cuuint64_t sstride = n_streams > 1 && !shared ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
     const cuuint64_t strides[3] = {(cuuint64_t)a.P * 8, (cuuint64_t)a.P * 8 * ROWS_BOX, sstride};
     const cuuint32_t box[4] = {(cuuint32_t)G, (cuuint32_t)ROWS_BOX, (cuuint32_t)(K2 / ROWS_BOX), 1};
     const cuuint32_t estr[4] = {1, 1, 1, 1};
     const CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT64, 4, const_cast<void*>(a.in), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
-    if (G == 10) return launch_g<10>(n_streams, a, tm, st);
+    if (G == 10) return launch_g<10>(n_streams, a, tm, shared, st);
     return cudaErrorInvalidValue;
 }
 

@@ -336,6 +336,51 @@ impl<Flt: GpuFloat> Chain<Flt> {
         Ok(Pushed { count, sample_rate: rate })
     }
 
+    /// A channelizer's push: every stream reads the same `chunk_len * n_chunks` samples of `input` (one wideband
+    /// row, copied to the device once), each with its own shift and state; `output` receives stream `s` at
+    /// `s * out_stride`.  Asynchronous when both are pinned: call [`Chain::sync`] before reading `output` or
+    /// modifying `input`.
+    pub fn push_shared(
+        &mut self,
+        sample_rate: f64,
+        chunk_len: usize,
+        n_chunks: usize,
+        input: &[Complex<Flt>],
+        output: &mut [Complex<Flt>],
+        out_stride: usize,
+    ) -> Result<Pushed, Error> {
+        assert!(input.len() >= chunk_len * n_chunks, "input slice too short");
+        let out_capacity = if self.n_streams > 1 { out_stride.min(output.len() - (self.n_streams - 1) * out_stride) } else { output.len() };
+        let (mut count, mut rate) = (0usize, 0f64);
+        check(unsafe {
+            sys::rr_chain_push_shared(
+                self.raw, sample_rate, chunk_len, n_chunks, input.as_ptr() as *const c_void, output.as_mut_ptr() as *mut c_void,
+                out_capacity, out_stride, &mut count, &mut rate,
+            )
+        })?;
+        Ok(Pushed { count, sample_rate: rate })
+    }
+
+    /// The same with device pointers: every stream reads the row at `dev_in` in place
+    ///
+    /// # Safety
+    /// `dev_in` must be a device allocation of the chain's device holding `chunk_len * n_chunks` complex samples,
+    /// `dev_out` one holding `n_streams` rows of `out_stride` complex samples.
+    pub unsafe fn push_shared_device(
+        &mut self,
+        sample_rate: f64,
+        chunk_len: usize,
+        n_chunks: usize,
+        dev_in: *const c_void,
+        dev_out: *mut c_void,
+        out_capacity: usize,
+        out_stride: usize,
+    ) -> Result<Pushed, Error> {
+        let (mut count, mut rate) = (0usize, 0f64);
+        check(sys::rr_chain_push_shared_device(self.raw, sample_rate, chunk_len, n_chunks, dev_in, dev_out, out_capacity, out_stride, &mut count, &mut rate))?;
+        Ok(Pushed { count, sample_rate: rate })
+    }
+
     /// Wait for everything enqueued by earlier pushes
     pub fn sync(&mut self) -> Result<(), Error> {
         check(unsafe { sys::rr_chain_sync(self.raw) })
