@@ -1086,8 +1086,7 @@ template <typename T> int poly_prepare(rr_chain* c, Stage& f, Stage& ds) {
     const size_t tab_bytes = (size_t)(Q * P) * (size_t)bestK * 2 * sizeof(T);
     if (tab_bytes > ((size_t)512 << 20)) return RR_OK;
     const double e8 = (double)P / (8.0 * (double)((P + 7) / 8)), e10 = (double)P / (10.0 * (double)((P + 9) / 10));
-    int G = e10 > e8 + 1e-9 ? 10 : 8;
-    if (const char* e = std::getenv("RR_POLY_G")) G = std::atoi(e) == 8 ? 8 : 10;
+    const int G = e10 > e8 + 1e-9 ? 10 : 8;
     if (!rr::poly_supported<T>(bestK, (int)Q, G)) return RR_OK;
     if (rr::poly_smem_bytes<T>(bestK, (int)Q, G, 1) > (size_t)220 * 1024) return RR_OK;
     std::vector<std::complex<double>> tab, perm;
@@ -1133,12 +1132,10 @@ template <typename T> int poly_prepare(rr_chain* c, Stage& f, Stage& ds) {
         const int cols = rank <= kFrontQRank ? kFrontQRank : RMAX;
         const bool narrow = cols == kFrontQRank && rr::front_supported(kFrontQRank, P);
         if (rank > 0 && lmq == (int)Lmax && (narrow || rr::front_wide_supported(cols, P))) {
-            std::vector<float> ac((size_t)P * cols);
+            std::vector<double> ac((size_t)P * cols);
             for (long long p = 0; p < P; ++p)
-                for (int cc = 0; cc < cols; ++cc) ac[(size_t)p * cols + cc] = (float)acf[(size_t)p * RMAX + cc];
-            RR_TRY(ds.acoef_q.ensure(ac.size() * sizeof(float)));
-            RR_CUDA(cudaMemcpyAsync(ds.acoef_q.p, ac.data(), ac.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-            RR_CUDA(cudaStreamSynchronize(c->stream));  // `ac` is pageable and dies here
+                for (int cc = 0; cc < cols; ++cc) ac[(size_t)p * cols + cc] = acf[(size_t)p * RMAX + cc];
+            RR_TRY(upload_real<float>(ds.acoef_q, ac, c->stream));
             constexpr int GQ = 8;
             const long long NRq = cols / GQ;
             perm.assign((size_t)(Q * NRq) * (size_t)bestK * (size_t)GQ, std::complex<double>(0.0, 0.0));
@@ -1188,12 +1185,10 @@ template <typename T> int poly_prepare(rr_chain* c, Stage& f, Stage& ds) {
             double disc = 0.0;
             const int lm2 = rr::design_rank_tables(f.taps, ds.ir_host_flt, P, K2, 2.0e-8, RK, &rank, &acf, &bfft, &disc);
             if (rank > 0 && lm2 == (int)Lmax) {
-                std::vector<float> ac((size_t)P * RK);
+                std::vector<double> ac((size_t)P * RK);
                 for (long long p = 0; p < P; ++p)
-                    for (int cc = 0; cc < RK; ++cc) ac[(size_t)(((p / 2) * 2 + (p & 1)) * RK + cc)] = (float)acf[(size_t)p * RK + cc];
-                RR_TRY(ds.acoef.ensure(ac.size() * sizeof(float)));
-                RR_CUDA(cudaMemcpyAsync(ds.acoef.p, ac.data(), ac.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-                RR_CUDA(cudaStreamSynchronize(c->stream));
+                    for (int cc = 0; cc < RK; ++cc) ac[(size_t)(((p / 2) * 2 + (p & 1)) * RK + cc)] = acf[(size_t)p * RK + cc];
+                RR_TRY(upload_real<float>(ds.acoef, ac, c->stream));
                 perm.assign((size_t)K2 * (size_t)RK, std::complex<double>(0.0, 0.0));
                 for (int cc = 0; cc < RK; ++cc)
                     for (int k = 0; k < K2; ++k) perm[(size_t)rr::poly2_table_index(RK, 0, cc, k)] = bfft[(size_t)cc * K2 + k] * scale2;
@@ -1205,8 +1200,7 @@ template <typename T> int poly_prepare(rr_chain* c, Stage& f, Stage& ds) {
                 if (c->allow_fused && rr::fused_supported(RK, P, (int)Lmax)) {
                     const int slot = fused_slot_acquire(c->ctx->device, &ds);
                     if (slot >= 0) {
-                        RR_CUDA(rr::fused_upload_coef(slot, ac.data(), (int)P, c->stream));
-                        RR_CUDA(cudaStreamSynchronize(c->stream));  // `ac` is pageable and dies here
+                        RR_CUDA(rr::fused_upload_coef(slot, (const float*)ds.acoef.p, (int)P, c->stream));
                         ds.fused_slot = slot;
                         ds.fused_valid = true;
                     }
@@ -1290,6 +1284,365 @@ struct DirectOut {
     long long user_stride = 0;
     bool done = false;
 };
+
+// ---- the polyphase part of run_filter_down ----------------------------------------------------------------------
+// What its routes share: the chunks [ca, n_chunks) of the push, whose filter outputs fire the Downsampler's outputs
+// m_lo..m_hi (1-based, counted with the reduced counters).  Filter output k aligns with push sample k; the kernels
+// read the (mixed on the fly) push chunks before the part, or hist2 below offset 0.
+struct PolyPart {
+    rr_chain* c;
+    Stage& f;
+    Stage& ds;
+    const FilterIo& io;
+    const StageAct& da;
+    DirectOut* direct;
+    long long P, Q;       // in/out = P/Q reduced
+    long long J0, m0;     // decimator counters referred to push sample 0 (J0 may be negative)
+    long long m_lo, m_hi;
+    long long I_lo, I_hi;  // low-rate indices of outputs m_lo and m_hi
+    long long len, n;     // pushed samples per stream, Filter chunk length
+    const rr::NcoStream* nco;
+    void* obase;          // output m goes to obase[m - m0 - 1] (rows ostride apart)
+    long long ostride;
+    bool tma_ok;          // (complex f32) the pushed samples can be read by TMA: rr::tma_input_ok
+    bool whole;           // the whole push is polyphase (no stateful chunks in front)
+    bool kept;            // whole, and the u rows the previous push kept are usable
+};
+
+// The Filter's next history is the last 2n mixed samples of the push, from push offset len - 2n.  A front end whose
+// rows cover push offsets [cover_lo, cover_hi) writes it, from max(len - 2n, 0) up to its last row, when those rows
+// reach back to that start; k_hist2_update copies the rest (Stage::hist_fused_*).  (A push shorter than 2n keeps the
+// end of the old history in front: those entries, [0, 2n - len), are always k_hist2_update's.)
+template <typename A> bool next_history(const PolyPart& p, long long cover_lo, long long cover_hi, A* a) {
+    Stage& f = p.f;
+    f.hist_fused_jlo = -1;
+    f.hist_fused_jfirst = 0;
+    const long long hfrom = p.len - 2 * p.n, hstart = std::max<long long>(hfrom, 0);
+    if (cover_lo > hstart || cover_hi <= hstart) return false;
+    a->hist_out = f.hist2[f.hist_cur ^ 1].p;
+    a->hist_from = hfrom;
+    a->hist_stride = 2 * p.n;
+    f.hist_fused_jlo = cover_hi - hfrom;
+    f.hist_fused_jfirst = hstart - hfrom;
+    return true;
+}
+
+// Direct output (complex f32): new output o lands at emitted position pending_before + o, so the outputs that complete
+// the caller's chunks go to the caller's buffer and the ones behind them (from out_split) to the other obuf
+template <typename A> void direct_split(const PolyPart& p, A* a) {
+    const long long emit = (long long)p.da.out.len();
+    if (!p.direct || !p.direct->user_out || emit < (long long)p.da.pending_before || emit <= 0) return;
+    a->out = (char*)p.direct->user_out + p.da.pending_before * 2 * sizeof(float);
+    a->out_stride = p.direct->user_stride;
+    a->out2 = p.ds.obuf[p.ds.obuf_cur ^ 1].p;
+    a->out2_stride = p.ostride;
+    a->out_split = emit - (long long)p.da.pending_before;
+    p.direct->done = true;
+}
+
+// k_poly2 blocks per group (one round of inverse transforms; bounded by shared memory) and groups per CTA half: as many
+// as keep the grid at two CTAs per SM or more, balanced
+void poly2_grid(rr::PolyArgs<float>* a, int G, int S, int sm_count) {
+    int nbpc = std::min(G, a->n_blocks);
+    while (nbpc > 1 && rr::poly2_smem_bytes(G, nbpc) > (size_t)226 * 1024) --nbpc;
+    const long long ctas_y = (S + 1) / 2;
+    while (nbpc > 1 && ctas_y * ((a->n_blocks + nbpc - 1) / nbpc) < 2LL * sm_count) --nbpc;
+    const int ngroups = (a->n_blocks + nbpc - 1) / nbpc;
+    a->nbpc = (a->n_blocks + ngroups - 1) / ngroups;
+    int ngrp = ngroups;
+    while (ngrp > 1 && ctas_y * ((ngroups + ngrp - 1) / ngrp) < 2LL * sm_count) --ngrp;
+    a->ngrp = ngrp;
+}
+
+// k_poly blocks per CTA: from `start` down to what shared memory holds (their parked spectra) and what keeps the grid at
+// two CTAs per SM, balanced -- the per-CTA tables are built once and the inverse rounds fill up (measured on C1, 7 blocks
+// per stream: 1.93 / 1.74 / 1.66 ms with 1 / 2 / 7 blocks per CTA)
+template <typename T> int poly_nbpc(int K, int Q, int G, int S, int n_blocks, int start, int sm_count) {
+    int nbpc = start;
+    while (nbpc > 1 && rr::poly_smem_bytes<T>(K, Q, G, nbpc) > (size_t)200 * 1024) --nbpc;
+    while (nbpc > 1 && (long long)S * ((n_blocks + nbpc - 1) / nbpc) < 2LL * sm_count) --nbpc;
+    const int nsb = (n_blocks + nbpc - 1) / nbpc;
+    return (n_blocks + nsb - 1) / nsb;
+}
+
+// the front ends' rows row_first .. row_first + n_rows - 1 of every stream to u, and the part of the Filter's next
+// history that rows up to push offset cover_hi reach
+rr::FrontArgs front_args(const PolyPart& p, const DevBuf& acoef, long long row_first, long long n_rows, void* u, long long u_stride,
+                         long long cover_hi) {
+    rr::FrontArgs fa{};
+    fa.in = p.io.in;
+    fa.in_stride = p.io.in_stride;
+    fa.len = p.len;
+    fa.hist2 = p.f.hist2[p.f.hist_cur].p;
+    fa.n = p.n;
+    fa.nco = p.nco;
+    fa.acoef = (const float*)acoef.p;
+    fa.P = (int)p.P;
+    fa.J0 = p.J0;
+    fa.row_first = row_first;
+    fa.n_rows = (int)n_rows;
+    fa.u = u;
+    fa.u_stride = u_stride;
+    fa.hist_staged = next_history(p, row_first * p.P - p.J0, cover_hi, &fa) && p.len < 4 * p.n;  // measured: pays off up to 3 chunks per push
+    return fa;
+}
+
+// the k_poly / k_poly2 arguments of the polyphase chain on the input itself
+template <typename T> rr::PolyArgs<T> input_poly_args(const PolyPart& p) {
+    rr::PolyArgs<T> a{};
+    a.in = p.io.in;
+    a.in_stride = p.io.in_stride;
+    a.len = p.len;
+    a.hist2 = p.f.hist2[p.f.hist_cur].p;
+    a.n = p.n;
+    a.nco = p.nco;
+    a.gtab = p.ds.gtab.p;
+    a.twK = p.ds.twK.p;
+    a.P = p.P;
+    a.Q = p.Q;
+    a.Lmax = p.ds.poly_Lmax;
+    a.V = p.ds.poly_V;
+    a.J0 = p.J0;
+    a.m0 = p.m0;
+    a.m_lo = p.m_lo;
+    a.m_hi = p.m_hi;
+    a.I_lo = p.I_lo;
+    a.out = p.obase;
+    a.out_stride = p.ostride;
+    return a;
+}
+
+// The routes, tried in this order by run_filter_down.  Each checks its preconditions first; when they hold it launches
+// its kernels and names itself in *route, else it leaves *route unset and the next route is tried.
+
+// k_fused: front end + low-rate part in one persistent kernel (u stays in shared memory).  Steady state only: the whole
+// push is polyphase, the previous push left its last Lmax rows of u behind, and there are enough streams to give every
+// SM whole streams; everything else takes k_front + k_poly2.
+int route_fused(const PolyPart& p, const char** route) {
+    rr_chain* c = p.c;
+    Stage& ds = p.ds;
+    const long long n_out = p.m_hi - p.m_lo + 1;
+    if (!(ds.poly2_valid && ds.front_valid && ds.fused_valid && c->allow_fused && p.tma_ok && p.kept && ds.ucache_ptr && p.Q == 1 &&
+          p.m0 == 0 && p.J0 >= 0 && p.J0 < p.P && c->S >= c->fused_min_streams && n_out >= c->fused_min_rows && p.len >= 33 * p.P))
+        return RR_OK;
+    constexpr int RK = 10;
+    const long long Lh = ds.poly_Lmax;
+    DevBuf& kb = ds.ukeep[ds.ukeep_cur];
+    RR_TRY(kb.ensure((size_t)c->S * (size_t)Lh * RK * 2 * sizeof(float)));
+    rr::FusedArgs fu{};
+    fu.in = p.io.in;
+    fu.in_stride = p.io.in_stride;
+    fu.len = p.len;
+    fu.hist2 = p.f.hist2[p.f.hist_cur].p;
+    fu.n = p.n;
+    fu.nco = p.nco;
+    fu.P = (int)p.P;
+    fu.coef_slot = ds.fused_slot;
+    fu.J0 = p.J0;
+    fu.n_out = (int)n_out;
+    fu.Lmax = (int)Lh;
+    fu.V = ds.poly2_V;
+    fu.ukeep_in = ds.ucache_ptr;
+    fu.ukeep_in_stride = ds.ucache_stride;
+    fu.ukeep_out = kb.p;
+    fu.ukeep_out_stride = Lh * RK;
+    fu.gtab = ds.gtab3.p;
+    fu.twK = ds.poly2_tw_own ? ds.twK2.p : ds.twK.p;
+    fu.out = p.obase;
+    fu.out_stride = p.ostride;
+    direct_split(p, &fu);
+    // the rows cover push offsets [-J0, m_hi*P - J0)
+    next_history(p, -p.J0, p.m_hi * p.P - p.J0, &fu);
+    RR_TIMED_LAUNCH(c, "k_fused", 1, rr::launch_fused(c->S, fu, p.io.shared, c->ctx->sm_count, c->stream));
+    ds.ucache_valid = true;
+    ds.ucache_rows = n_out + Lh;
+    ds.ucache_ptr = kb.p;
+    ds.ucache_stride = Lh * RK;
+    ds.ukeep_cur ^= 1;
+    *route = "fused[filter+down]";
+    return RR_OK;
+}
+
+// k_front + k_poly2 (Q == 1, the filter factors to rank 10): u rows [m_lo-1-Lmax, m_hi-1] of every stream, then the
+// low-rate part on u as a stream of RK branches whose first output (virtual index Lmax+1) is output m_lo
+int route_front_poly2(const PolyPart& p, const char** route) {
+    rr_chain* c = p.c;
+    Stage& ds = p.ds;
+    if (!(ds.poly2_valid && ds.front_valid && p.tma_ok)) return RR_OK;
+    constexpr int RK = 10;
+    const int S = c->S;
+    const long long Lh = ds.poly_Lmax;
+    const long long n_out = p.m_hi - p.m_lo + 1;
+    const long long n_rows = n_out + Lh;
+    if (n_rows >= (1LL << 27)) return RR_OK;
+    // every stream's rows are followed by one transform length of zero rows, so that the low-rate part
+    // reads whole tiles by TMA up to and including its last block (no edge path, no shifted block)
+    // (rows beyond n_rows only feed outputs that are not stored; the stride is rounded so that pushes whose
+    // output count differs by a few keep the layout, and what an earlier push left there is that stream's own)
+    const long long pad_rows = 512;
+    const long long u_stride = (((n_rows + 127) / 128 * 128 + pad_rows) * RK + 1) / 2 * 2;
+    // short pushes (one block per stream): the low-rate part takes runs of sab_nb streams as the blocks of
+    // one "stream", so that an inverse round serves several streams (PolyArgs::sab_*)
+    const int n_blocks1 = (int)((n_out - 1) / ds.poly2_V + 1);
+    const int halves_total = 2 * c->ctx->sm_count;
+    const int sab_run = (c->allow_sab && n_blocks1 <= 3 && S > halves_total) ? (S + halves_total - 1) / halves_total : 0;  // streams
+    const int sab_nb = sab_run * n_blocks1;  // blocks of a run
+    const size_t S_alloc = sab_run ? (size_t)((S + sab_run - 1) / sab_run) * sab_run : (size_t)S;
+    const size_t ubytes = S_alloc * (size_t)u_stride * 2 * sizeof(float);
+    DevBuf& ub = ds.ubuf[ds.ubuf_cur];
+    if (ub.bytes < ubytes || ds.ubuf_stride[ds.ubuf_cur] != u_stride) {
+        // a new layout: the pad rows must read as zeros (they only ever feed outputs that are not stored,
+        // but a NaN there would spread through the transform)
+        RR_TRY(ub.ensure(ubytes));
+        RR_CUDA(cudaMemsetAsync(ub.p, 0, ubytes, c->stream));
+        ds.ubuf_stride[ds.ubuf_cur] = u_stride;
+    }
+    // history rows: kept from the previous push when it went through here too (k_front moves them over itself), else
+    // recomputed from hist2
+    const bool cached = p.kept && ds.ucache_rows >= Lh && n_out > 0;
+    rr::FrontArgs fa = front_args(p, ds.acoef, p.m_lo - 1 - (cached ? 0 : Lh), cached ? n_out : n_rows,
+                                  (char*)ub.p + (cached ? (size_t)Lh * RK * 2 * sizeof(float) : 0), u_stride, p.m_hi * p.P - p.J0);
+    if (cached) {
+        fa.kept_src = ds.ucache_ptr;
+        fa.kept_stride = ds.ucache_stride;
+        fa.kept_rows = (int)Lh;
+    }
+    RR_TIMED_LAUNCH(c, "k_front", 1, rr::launch_front(RK, S, fa, p.io.shared, c->ctx->sm_count, c->stream));
+    rr::PolyArgs<float> b{};
+    b.in = ub.p;
+    b.in_stride = u_stride;
+    b.len = (n_rows + pad_rows) * RK;
+    b.hist2 = ub.p;
+    b.n = 0;
+    b.nco = nullptr;
+    b.gtab = ds.gtab3.p;
+    b.twK = ds.poly2_tw_own ? ds.twK2.p : ds.twK.p;
+    b.P = RK;
+    b.Q = 1;
+    b.Lmax = ds.poly_Lmax;
+    b.V = ds.poly2_V;
+    b.J0 = 0;
+    b.m0 = ds.poly_Lmax;
+    b.m_lo = ds.poly_Lmax + 1;
+    b.m_hi = ds.poly_Lmax + n_out;
+    b.I_lo = b.m_lo;
+    b.n_blocks = (int)((b.m_hi - b.I_lo) / b.V + 1);
+    poly2_grid(&b, RK, S, c->ctx->sm_count);
+    b.out = p.obase;
+    b.out_stride = p.ostride;
+    int S2 = S;  // streams of the low-rate launch
+    if (sab_nb) {
+        int nb2 = std::min(RK, sab_nb);
+        while (nb2 > 1 && rr::poly2_smem_bytes(RK, nb2) > (size_t)226 * 1024) --nb2;
+        const int groups2 = (sab_nb + nb2 - 1) / nb2;
+        b.n_blocks = sab_nb;
+        b.nbpc = (sab_nb + groups2 - 1) / groups2;
+        b.ngrp = groups2;  // a half takes all groups of its run of streams
+        b.sab_blocks = sab_nb;
+        b.sab_rb = n_blocks1;
+        b.sab_streams = S;
+        b.sab_in_step = u_stride;
+        b.in_stride = (long long)sab_run * u_stride;
+        b.len = (long long)sab_run * u_stride;
+        S2 = (S + sab_run - 1) / sab_run;
+    }
+    if (p.whole) direct_split(p, &b);
+    if (sab_nb) {
+        b.sab_out_step = b.out_stride;
+        b.sab_out2_step = b.out2_stride;
+        b.out_stride *= sab_run;
+        b.out2_stride *= sab_run;
+    }
+    RR_TIMED_LAUNCH(c, "k_poly2", 1, rr::launch_poly2(RK, S2, b, false, c->ctx->sm_count, c->stream));
+    ds.ucache_valid = true;
+    ds.ucache_rows = n_rows;
+    // the last Lmax rows of [history rows | new rows] of this push
+    ds.ucache_ptr = (const char*)ub.p + (size_t)(n_rows - Lh) * RK * 2 * sizeof(float);
+    ds.ucache_stride = u_stride;
+    ds.ubuf_cur ^= 1;
+    *route = "front+poly2[filter+down]";
+    return RR_OK;
+}
+
+// k_front / k_front_wide + k_poly (Q > 1): u rows [I_lo-1-Lmax, I_hi] (tap l = -1 of the phases q > 0 reads row I),
+// then k_poly on u with the Q phase tables.  Output m = Q*I + q keeps its index: block 0's window starts at u row 0,
+// which is row I_lo-1-Lmax of the stream (PolyArgs::J0 in units of u samples).  No rows are kept between pushes (the
+// last row of a push is cut off by its end).
+int route_front_q(const PolyPart& p, const char** route) {
+    rr_chain* c = p.c;
+    Stage& ds = p.ds;
+    if (!(ds.frontq_valid && (p.tma_ok || ds.frontq_wide) && p.Q > 1)) return RR_OK;
+    const int S = c->S;
+    const int RQ = ds.frontq_cols;
+    constexpr int GQ = 8;
+    const long long Lh = ds.poly_Lmax;
+    const long long row_first = p.I_lo - 1 - Lh;
+    const long long n_rows = p.I_hi - p.I_lo + 2 + Lh;
+    const long long u_stride = n_rows * RQ;
+    if (n_rows * p.P >= (1LL << 31)) return RR_OK;
+    DevBuf& ub = ds.ubuf[0];
+    RR_TRY(ub.ensure((size_t)S * (size_t)u_stride * 2 * sizeof(float)));
+    ds.ubuf_stride[0] = -1;
+    // the rows cover push offsets up to (I_hi+1)*P - J0, cut off at the end of the push
+    const rr::FrontArgs fa = front_args(p, ds.acoef_q, row_first, n_rows, ub.p, u_stride, std::min<long long>((p.I_hi + 1) * p.P - p.J0, p.len));
+    if (ds.frontq_wide) RR_TIMED_LAUNCH(c, "k_front_wide", 1, rr::launch_front_wide(RQ, S, fa, c->stream));
+    else RR_TIMED_LAUNCH(c, "k_front", 1, rr::launch_front(RQ, S, fa, p.io.shared, c->ctx->sm_count, c->stream));
+    rr::PolyArgs<float> b{};
+    b.in = ub.p;
+    b.in_stride = u_stride;
+    b.len = n_rows * RQ;
+    b.hist2 = ub.p;
+    b.n = 0;
+    b.nco = nullptr;
+    b.gtab = ds.gtab_q.p;
+    b.twK = ds.twK.p;
+    b.P = RQ;
+    b.Q = p.Q;
+    b.Lmax = (int)Lh;
+    b.V = ds.poly_V;
+    b.J0 = row_first * RQ;
+    b.m0 = p.m0;
+    b.m_lo = p.m_lo;
+    b.m_hi = p.m_hi;
+    b.I_lo = p.I_lo;
+    b.n_blocks = (int)((p.I_hi - p.I_lo) / b.V + 1);
+    b.nbpc = poly_nbpc<float>(ds.poly_K, (int)p.Q, GQ, S, b.n_blocks, b.n_blocks, c->ctx->sm_count);
+    b.out = p.obase;
+    b.out_stride = p.ostride;
+    RR_TIMED_LAUNCH(c, "k_poly(u)", 1, rr::launch_poly<float>(ds.poly_K, (int)p.Q, GQ, S, b, c->stream));
+    *route = "front+poly[filter+down]";
+    return RR_OK;
+}
+
+// k_poly2 on all P branches of the input (Q == 1, a filter that does not factor to rank 10)
+int route_poly2(const PolyPart& p, const char** route) {
+    rr_chain* c = p.c;
+    Stage& ds = p.ds;
+    if (!(ds.poly2_valid && p.tma_ok)) return RR_OK;
+    rr::PolyArgs<float> a = input_poly_args<float>(p);
+    a.gtab = ds.gtab2.p;
+    if (ds.poly2_tw_own) a.twK = ds.twK2.p;
+    a.V = ds.poly2_V;
+    a.n_blocks = (int)((p.I_hi - p.I_lo) / a.V + 1);
+    poly2_grid(&a, ds.poly2_G, c->S, c->ctx->sm_count);
+    RR_TIMED_LAUNCH(c, "k_poly2", 1, rr::launch_poly2(ds.poly2_G, c->S, a, p.io.shared, c->ctx->sm_count, c->stream));
+    *route = "poly2[filter+down]";
+    return RR_OK;
+}
+
+// k_poly: the generic polyphase kernel (f32 and f64, any Q <= 4); blocks per CTA start at one round of inverse
+// transforms (G jobs)
+template <typename T> int route_poly(const PolyPart& p, const char** route) {
+    rr_chain* c = p.c;
+    Stage& ds = p.ds;
+    rr::PolyArgs<T> a = input_poly_args<T>(p);
+    a.n_blocks = (int)((p.I_hi - p.I_lo) / a.V + 1);
+    a.nbpc = poly_nbpc<T>(ds.poly_K, (int)p.Q, ds.poly_G, c->S, a.n_blocks, std::max(1, ds.poly_G / (int)p.Q), c->ctx->sm_count);
+    RR_TIMED_LAUNCH(c, "k_poly", 1, rr::launch_poly<T>(ds.poly_K, (int)p.Q, ds.poly_G, c->S, a, c->stream));
+    *route = "poly[filter+down]";
+    return RR_OK;
+}
+
 template <typename T>
 int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const StageAct& fa, const StageAct& da, std::string* plan,
                     DirectOut* direct = nullptr) {
@@ -1372,373 +1725,27 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
         j0 = (j0 + zlen) % ds.h.P;
         m0 = floordiv128(j0, ds.h.Q, ds.h.P);
     }
+    if (ca == io.n_chunks) return RR_OK;
 
     // ---- polyphase part: chunks [ca, n_chunks) ----------------------------------------
-    if (ca < io.n_chunks) {
-        const long long Pq = ds.h.P, Qq = ds.h.Q;
-        const long long zlen = (long long)((io.n_chunks - ca) * n);  // filter outputs covered by this part
-        // outputs m (1-based, counted with the reduced counters) firing inside this part
-        const long long m_lo = m0 + 1;
-        const long long m_hi = floordiv128(j0 + zlen, Qq, Pq);
-        bool used_poly2 = false, used_front = false, used_fused = false, used_frontq = false;
-        if (m_hi >= m_lo) {
-            rr::PolyArgs<T> a{};
-            // filter output k aligns with push sample k; the part starts at push sample ca*n, and the
-            // kernel reads the (mixed on the fly) push chunks before it, or hist2 below offset 0
-            a.in = io.in;
-            a.in_stride = io.in_stride;
-            a.len = (long long)(io.n_chunks * n);
-            a.n = (long long)n;
-            a.nco = io.nco ? (const rr::NcoStream*)io.nco->nco_d.p : nullptr;
-            a.gtab = ds.gtab.p;
-            a.twK = ds.twK.p;
-            a.P = Pq;
-            a.Q = Qq;
-            a.Lmax = ds.poly_Lmax;
-            a.V = ds.poly_V;
-            a.J0 = j0 - (long long)(ca * n);  // counters referred to push sample 0 (may be negative)
-            a.m0 = m0;
-            a.m_lo = m_lo;
-            a.m_hi = m_hi;
-            a.I_lo = m_lo / Qq;
-            const long long I_hi = m_hi / Qq;
-            bool done = false;
-            if constexpr (std::is_same<T, float>::value) {
-                const bool tma_ok = ((uintptr_t)a.in % 16 == 0) && (S == 1 || io.shared || a.in_stride % 2 == 0) && a.len < (1LL << 31);
-                // ---- k_fused: front end + low-rate part in one persistent kernel (u stays in shared memory).  Steady
-                // state only: the whole push is polyphase, the previous push left its last Lmax rows of u behind, and
-                // there are enough streams to give every SM whole streams; everything else takes k_front + k_poly2.
-                if (ds.poly2_valid && ds.front_valid && ds.fused_valid && c->allow_fused && tma_ok && ca == 0 && was_ucache_valid &&
-                    c->allow_ucache && ds.ucache_ptr && Qq == 1 && m0 == 0 && a.J0 >= 0 && a.J0 < Pq && S >= c->fused_min_streams &&
-                    m_hi - m_lo + 1 >= c->fused_min_rows && a.len >= 33 * Pq) {
-                    constexpr int RK = 10;
-                    const long long n_out = m_hi - m_lo + 1;
-                    const long long Lh = ds.poly_Lmax;
-                    const size_t kbytes = (size_t)S * (size_t)Lh * RK * 2 * sizeof(float);
-                    DevBuf& kb = ds.ukeep[ds.ukeep_cur];
-                    RR_TRY(kb.ensure(kbytes));
-                    rr::FusedArgs fu{};
-                    fu.in = a.in;
-                    fu.in_stride = a.in_stride;
-                    fu.len = a.len;
-                    fu.hist2 = f.hist2[f.hist_cur].p;
-                    fu.n = a.n;
-                    fu.nco = a.nco;
-                    fu.P = (int)Pq;
-                    fu.coef_slot = ds.fused_slot;
-                    fu.J0 = a.J0;
-                    fu.n_out = (int)n_out;
-                    fu.Lmax = (int)Lh;
-                    fu.V = ds.poly2_V;
-                    fu.ukeep_in = ds.ucache_ptr;
-                    fu.ukeep_in_stride = ds.ucache_stride;
-                    fu.ukeep_out = kb.p;
-                    fu.ukeep_out_stride = Lh * RK;
-                    fu.gtab = ds.gtab3.p;
-                    fu.twK = ds.poly2_tw_own ? ds.twK2.p : ds.twK.p;
-                    fu.out = obase;
-                    fu.out_stride = ostride;
-                    const long long emit = (long long)da.out.len();
-                    if (direct && direct->user_out && emit >= (long long)da.pending_before && emit > 0) {
-                        fu.out = (char*)direct->user_out + da.pending_before * 2 * sizeof(T);
-                        fu.out_stride = direct->user_stride;
-                        fu.out2 = ds.obuf[ds.obuf_cur ^ 1].p;
-                        fu.out2_stride = ostride;
-                        fu.out_split = emit - (long long)da.pending_before;
-                        direct->done = true;
-                    }
-                    // the rows cover push offsets [-J0, m_hi*P - J0): the kernel also writes the Filter's next history
-                    // from len - 2n up to its last row (the rest is k_hist2_update's)
-                    const long long cover_hi = m_hi * Pq - a.J0;
-                    f.hist_fused_jlo = -1;
-                    f.hist_fused_jfirst = 0;
-                    const long long hfrom = a.len - 2 * a.n, hstart = std::max<long long>(hfrom, 0);
-                    if (cover_hi > hstart) {
-                        fu.hist_out = f.hist2[f.hist_cur ^ 1].p;
-                        fu.hist_from = hfrom;
-                        fu.hist_stride = 2 * a.n;
-                        f.hist_fused_jlo = cover_hi - hfrom;
-                        f.hist_fused_jfirst = hstart - hfrom;
-                    }
-                    RR_TIMED_LAUNCH(c, "k_fused", 1, rr::launch_fused(S, fu, io.shared, c->ctx->sm_count, st));
-                    ds.ucache_valid = true;
-                    ds.ucache_rows = n_out + Lh;
-                    ds.ucache_ptr = kb.p;
-                    ds.ucache_stride = Lh * RK;
-                    ds.ukeep_cur ^= 1;
-                    done = true;
-                    used_fused = true;
-                }
-                if (!done && ds.poly2_valid && ds.front_valid && tma_ok) {
-                    // u rows [m_lo-1-Lmax, m_hi-1] of every stream, then the low-rate part on u as a stream of
-                    // RK branches whose first output (virtual index Lmax+1) is output m_lo
-                    constexpr int RK = 10;
-                    const int G2 = RK;
-                    const long long n_out = m_hi - m_lo + 1;
-                    const long long n_rows = n_out + ds.poly_Lmax;
-                    // every stream's rows are followed by one transform length of zero rows, so that the low-rate part
-                    // reads whole tiles by TMA up to and including its last block (no edge path, no shifted block)
-                    // (rows beyond n_rows only feed outputs that are not stored; the stride is rounded so that pushes whose
-                    // output count differs by a few keep the layout, and what an earlier push left there is that stream's own)
-                    const long long pad_rows = 512;
-                    const long long u_stride = (((n_rows + 127) / 128 * 128 + pad_rows) * RK + 1) / 2 * 2;
-                    if (n_rows < (1LL << 27)) {
-                        // short pushes (one block per stream): the low-rate part takes runs of sab_nb streams as the blocks of
-                        // one "stream", so that an inverse round serves several streams (PolyArgs::sab_*)
-                        const int n_blocks1 = (int)((n_out - 1) / ds.poly2_V + 1);
-                        const int halves_total = 2 * c->ctx->sm_count;
-                        const int sab_run = (c->allow_sab && n_blocks1 <= 3 && S > halves_total) ? (S + halves_total - 1) / halves_total : 0;  // streams
-                        const int sab_nb = sab_run * n_blocks1;  // blocks of a run
-                        const size_t S_alloc = sab_run ? (size_t)((S + sab_run - 1) / sab_run) * sab_run : (size_t)S;
-                        const size_t ubytes = S_alloc * (size_t)u_stride * 2 * sizeof(float);
-                        DevBuf& ub = ds.ubuf[ds.ubuf_cur];
-                        if (ub.bytes < ubytes || ds.ubuf_stride[ds.ubuf_cur] != u_stride) {
-                            // a new layout: the pad rows must read as zeros (they only ever feed outputs that are not stored,
-                            // but a NaN there would spread through the transform)
-                            RR_TRY(ub.ensure(ubytes));
-                            RR_CUDA(cudaMemsetAsync(ub.p, 0, ubytes, st));
-                            ds.ubuf_stride[ds.ubuf_cur] = u_stride;
-                        }
-                        // history rows: kept from the previous push when it went through here too, else recomputed from hist2
-                        const long long Lh = ds.poly_Lmax;
-                        const bool cached = was_ucache_valid && c->allow_ucache && ca == 0 && ds.ucache_rows >= Lh && n_out > 0;
-                        rr::FrontArgs fa{};
-                        if (cached) {  // k_front moves them over itself
-                            fa.kept_src = ds.ucache_ptr;
-                            fa.kept_stride = ds.ucache_stride;
-                            fa.kept_rows = (int)Lh;
-                        }
-                        fa.in = a.in;
-                        fa.in_stride = a.in_stride;
-                        fa.len = a.len;
-                        fa.hist2 = f.hist2[f.hist_cur].p;
-                        fa.n = a.n;
-                        fa.nco = a.nco;
-                        fa.acoef = (const float*)ds.acoef.p;
-                        fa.P = (int)Pq;
-                        fa.J0 = a.J0;
-                        fa.row_first = m_lo - 1 - (cached ? 0 : Lh);
-                        fa.n_rows = (int)(cached ? n_out : n_rows);
-                        fa.u = (char*)ub.p + (cached ? (size_t)Lh * RK * 2 * sizeof(float) : 0);
-                        fa.u_stride = u_stride;
-                        // the rows cover push offsets [row_first*P - J0, m_hi*P - J0): when that reaches back to
-                        // len - 2n the kernel also writes the Filter's next history up to its last row
-                        const long long cover_lo = fa.row_first * Pq - a.J0, cover_hi = m_hi * Pq - a.J0;
-                        f.hist_fused_jlo = -1;
-                        f.hist_fused_jfirst = 0;
-                        // (a push shorter than 2n keeps the end of the old history in front: those entries, [0, 2n - len),
-                        // are copied by k_hist2_update)
-                        const long long hfrom = a.len - 2 * a.n, hstart = std::max<long long>(hfrom, 0);
-                        if (cover_lo <= hstart && cover_hi > hstart) {
-                            fa.hist_out = f.hist2[f.hist_cur ^ 1].p;
-                            fa.hist_from = hfrom;
-                            fa.hist_stride = 2 * a.n;
-                            fa.hist_staged = a.len < 4 * a.n ? 1 : 0;  // measured: pays off up to 3 chunks per push
-                            f.hist_fused_jlo = cover_hi - hfrom;
-                            f.hist_fused_jfirst = hstart - hfrom;
-                        }
-                        RR_TIMED_LAUNCH(c, "k_front", 1, rr::launch_front(RK, S, fa, io.shared, st));
-                        rr::PolyArgs<float> b{};
-                        b.in = ub.p;
-                        b.in_stride = u_stride;
-                        b.len = (n_rows + pad_rows) * RK;
-                        b.hist2 = ub.p;
-                        b.n = 0;
-                        b.nco = nullptr;
-                        b.gtab = ds.gtab3.p;
-                        b.twK = ds.poly2_tw_own ? ds.twK2.p : ds.twK.p;
-                        b.P = RK;
-                        b.Q = 1;
-                        b.Lmax = ds.poly_Lmax;
-                        b.V = ds.poly2_V;
-                        b.J0 = 0;
-                        b.m0 = ds.poly_Lmax;
-                        b.m_lo = ds.poly_Lmax + 1;
-                        b.m_hi = ds.poly_Lmax + n_out;
-                        b.I_lo = b.m_lo;
-                        b.n_blocks = (int)((b.m_hi - b.I_lo) / b.V + 1);
-                        int nbpc = std::min(G2, b.n_blocks);
-                        while (nbpc > 1 && rr::poly2_smem_bytes(G2, nbpc) > (size_t)226 * 1024) --nbpc;
-                        const long long ctas_y = (S + 1) / 2;
-                        while (nbpc > 1 && ctas_y * ((b.n_blocks + nbpc - 1) / nbpc) < 2LL * c->ctx->sm_count) --nbpc;
-                        const int ngroups = (b.n_blocks + nbpc - 1) / nbpc;
-                        nbpc = (b.n_blocks + ngroups - 1) / ngroups;
-                        int ngrp = ngroups;
-                        while (ngrp > 1 && ctas_y * ((ngroups + ngrp - 1) / ngrp) < 2LL * c->ctx->sm_count) --ngrp;
-                        b.nbpc = nbpc;
-                        b.ngrp = ngrp;
-                        b.out = obase;
-                        b.out_stride = ostride;
-                        int S2 = S;  // streams of the low-rate launch
-                        if (sab_nb) {
-                            int nb2 = std::min(G2, sab_nb);
-                            while (nb2 > 1 && rr::poly2_smem_bytes(G2, nb2) > (size_t)226 * 1024) --nb2;
-                            const int groups2 = (sab_nb + nb2 - 1) / nb2;
-                            b.n_blocks = sab_nb;
-                            b.nbpc = (sab_nb + groups2 - 1) / groups2;
-                            b.ngrp = groups2;  // a half takes all groups of its run of streams
-                            b.sab_blocks = sab_nb;
-                            b.sab_rb = n_blocks1;
-                            b.sab_streams = S;
-                            b.sab_in_step = u_stride;
-                            b.in_stride = (long long)sab_run * u_stride;
-                            b.len = (long long)sab_run * u_stride;
-                            S2 = (S + sab_run - 1) / sab_run;
-                        }
-                        const long long emit = (long long)da.out.len();
-                        if (direct && direct->user_out && ca == 0 && emit >= (long long)da.pending_before && emit > 0) {
-                            // new output o lands at emitted position pending_before + o
-                            b.out = (char*)direct->user_out + da.pending_before * 2 * sizeof(T);
-                            b.out_stride = direct->user_stride;
-                            b.out2 = ds.obuf[ds.obuf_cur ^ 1].p;
-                            b.out2_stride = ostride;
-                            b.out_split = emit - (long long)da.pending_before;
-                            direct->done = true;
-                        }
-                        if (sab_nb) {
-                            b.sab_out_step = b.out_stride;
-                            b.sab_out2_step = b.out2_stride;
-                            b.out_stride *= sab_run;
-                            b.out2_stride *= sab_run;
-                        }
-                        RR_TIMED_LAUNCH(c, "k_poly2", 1, rr::launch_poly2(G2, S2, b, false, st));
-                        ds.ucache_valid = true;
-                        ds.ucache_rows = n_rows;
-                        // the last Lmax rows of [history rows | new rows] of this push
-                        ds.ucache_ptr = (const char*)ub.p + (size_t)(n_rows - Lh) * RK * 2 * sizeof(float);
-                        ds.ucache_stride = u_stride;
-                        ds.ubuf_cur ^= 1;
-                        done = true;
-                        used_front = true;
-                    }
-                }
-                if (!done && ds.frontq_valid && (tma_ok || ds.frontq_wide) && Qq > 1) {
-                    // Q > 1: u rows [I_first-1-Lmax, I_last] (tap l = -1 of the phases q > 0 reads row I), then k_poly on u with
-                    // the Q phase tables.  Output m = Q*I + q keeps its index: block 0's window starts at u row 0, which is
-                    // row I_first-1-Lmax of the stream (PolyArgs::J0 in units of u samples).  No rows are kept between pushes
-                    // (the last row of a push is cut off by its end), the Filter's history is k_hist2_update's.
-                    const int RQ = ds.frontq_cols;
-                    constexpr int GQ = 8;
-                    const long long Lh = ds.poly_Lmax;
-                    const long long I_first = a.I_lo, I_last = I_hi;
-                    const long long row_first = I_first - 1 - Lh;
-                    const long long n_rows = I_last - I_first + 2 + Lh;
-                    const long long u_stride = n_rows * RQ;
-                    if (n_rows * Pq < (1LL << 31)) {
-                        DevBuf& ub = ds.ubuf[0];
-                        RR_TRY(ub.ensure((size_t)S * (size_t)u_stride * 2 * sizeof(float)));
-                        ds.ubuf_stride[0] = -1;
-                        rr::FrontArgs fa{};
-                        fa.in = a.in;
-                        fa.in_stride = a.in_stride;
-                        fa.len = a.len;
-                        fa.hist2 = f.hist2[f.hist_cur].p;
-                        fa.n = a.n;
-                        fa.nco = a.nco;
-                        fa.acoef = (const float*)ds.acoef_q.p;
-                        fa.P = (int)Pq;
-                        fa.J0 = a.J0;
-                        fa.row_first = row_first;
-                        fa.n_rows = (int)n_rows;
-                        fa.u = ub.p;
-                        fa.u_stride = u_stride;
-                        // the rows cover push offsets [row_first*P - J0, (I_last+1)*P - J0), cut off at the end of the push: when
-                        // that reaches back to len - 2n the kernel also writes the Filter's next history
-                        const long long cover_lo = row_first * Pq - a.J0, cover_hi = std::min<long long>((I_last + 1) * Pq - a.J0, a.len);
-                        f.hist_fused_jlo = -1;
-                        f.hist_fused_jfirst = 0;
-                        const long long hfrom = a.len - 2 * a.n, hstart = std::max<long long>(hfrom, 0);
-                        if (cover_lo <= hstart && cover_hi > hstart) {
-                            fa.hist_out = f.hist2[f.hist_cur ^ 1].p;
-                            fa.hist_from = hfrom;
-                            fa.hist_stride = 2 * a.n;
-                            fa.hist_staged = a.len < 4 * a.n ? 1 : 0;
-                            f.hist_fused_jlo = cover_hi - hfrom;
-                            f.hist_fused_jfirst = hstart - hfrom;
-                        }
-                        if (ds.frontq_wide) RR_TIMED_LAUNCH(c, "k_front_wide", 1, rr::launch_front_wide(RQ, S, fa, st));
-                        else RR_TIMED_LAUNCH(c, "k_front", 1, rr::launch_front(RQ, S, fa, io.shared, st));
-                        rr::PolyArgs<float> b{};
-                        b.in = ub.p;
-                        b.in_stride = u_stride;
-                        b.len = n_rows * RQ;
-                        b.hist2 = ub.p;
-                        b.n = 0;
-                        b.nco = nullptr;
-                        b.gtab = ds.gtab_q.p;
-                        b.twK = ds.twK.p;
-                        b.P = RQ;
-                        b.Q = Qq;
-                        b.Lmax = (int)Lh;
-                        b.V = ds.poly_V;
-                        b.J0 = row_first * RQ;
-                        b.m0 = a.m0;
-                        b.m_lo = a.m_lo;
-                        b.m_hi = a.m_hi;
-                        b.I_lo = I_first;
-                        b.n_blocks = (int)((I_last - I_first) / b.V + 1);
-                        // blocks per CTA: as many as shared memory holds (their parked spectra) while the grid stays at two
-                        // CTAs per SM -- the per-CTA tables are built once and the inverse rounds fill up (measured on C1, 7
-                        // blocks per stream: 1.93 / 1.74 / 1.66 ms with 1 / 2 / 7 blocks per CTA)
-                        int nbpc = b.n_blocks;
-                        while (nbpc > 1 && rr::poly_smem_bytes<float>(ds.poly_K, (int)Qq, GQ, nbpc) > (size_t)200 * 1024) --nbpc;
-                        while (nbpc > 1 && (long long)S * ((b.n_blocks + nbpc - 1) / nbpc) < 2LL * c->ctx->sm_count) --nbpc;
-                        const int nsb = (b.n_blocks + nbpc - 1) / nbpc;
-                        b.nbpc = (b.n_blocks + nsb - 1) / nsb;
-                        b.out = obase;
-                        b.out_stride = ostride;
-                        RR_TIMED_LAUNCH(c, "k_poly(u)", 1, rr::launch_poly<float>(ds.poly_K, (int)Qq, GQ, S, b, st));
-                        done = true;
-                        used_frontq = true;
-                    }
-                }
-                if (!done && ds.poly2_valid && tma_ok) {
-                    a.gtab = ds.gtab2.p;
-                    if (ds.poly2_tw_own) a.twK = ds.twK2.p;
-                    a.V = ds.poly2_V;
-                    a.n_blocks = (int)((I_hi - a.I_lo) / a.V + 1);
-                    const int G2 = ds.poly2_G;
-                    // blocks per CTA: bounded by the columns that run the inverse transforms and by the
-                    // shared memory that lets two CTAs share an SM
-                    // blocks per group (one round of inverse transforms; bounded by shared memory), groups per
-                    // CTA half: as many as keep the grid at two CTAs per SM or more
-                    int nbpc = std::min(G2, a.n_blocks);
-                    while (nbpc > 1 && rr::poly2_smem_bytes(G2, nbpc) > (size_t)226 * 1024) --nbpc;
-                    const long long ctas_y = (S + 1) / 2;
-                    while (nbpc > 1 && ctas_y * ((a.n_blocks + nbpc - 1) / nbpc) < 2LL * c->ctx->sm_count) --nbpc;
-                    const int ngroups = (a.n_blocks + nbpc - 1) / nbpc;
-                    nbpc = (a.n_blocks + ngroups - 1) / ngroups;  // balance
-                    int ngrp = ngroups;
-                    while (ngrp > 1 && ctas_y * ((ngroups + ngrp - 1) / ngrp) < 2LL * c->ctx->sm_count) --ngrp;
-                    a.nbpc = nbpc;
-                    a.ngrp = ngrp;
-                    a.out = obase;
-                    a.out_stride = ostride;
-                    a.hist2 = f.hist2[f.hist_cur].p;
-                    RR_TIMED_LAUNCH(c, "k_poly2", 1, rr::launch_poly2(G2, S, a, io.shared, st));
-                    done = true;
-                    used_poly2 = true;
-                }
-            }
-            if (!done) {
-                a.n_blocks = (int)((I_hi - a.I_lo) / a.V + 1);
-                // blocks per CTA: one round of inverse transforms (G jobs) when the grid stays large enough
-                int nbpc = std::max(1, ds.poly_G / (int)Qq);
-                while (nbpc > 1 && rr::poly_smem_bytes<T>(ds.poly_K, (int)Qq, ds.poly_G, nbpc) > (size_t)200 * 1024) --nbpc;
-                while (nbpc > 1 && (long long)S * ((a.n_blocks + nbpc - 1) / nbpc) < 2LL * c->ctx->sm_count) --nbpc;
-                const int nsb = (a.n_blocks + nbpc - 1) / nbpc;
-                nbpc = (a.n_blocks + nsb - 1) / nsb;  // balance
-                a.nbpc = nbpc;
-                a.out = obase;
-                a.out_stride = ostride;
-                a.hist2 = f.hist2[f.hist_cur].p;
-                RR_TIMED_LAUNCH(c, "k_poly", 1, rr::launch_poly<T>(ds.poly_K, (int)Qq, ds.poly_G, S, a, st));
-            }
-        }
-        ds.ztail_stale = true;
-        if (!plan->empty() && plan->back() != '+' && plan->back() != '|' && ca > 0) *plan += "|";
-        *plan += used_frontq ? "front+poly[filter+down]" : used_fused ? "fused[filter+down]" : (used_front ? "front+poly2[filter+down]" : (used_poly2 ? "poly2[filter+down]" : "poly[filter+down]"));
+    const long long P = ds.h.P, Q = ds.h.Q, len = (long long)(io.n_chunks * n);
+    const long long m_lo = m0 + 1, m_hi = floordiv128(j0 + (long long)((io.n_chunks - ca) * n), Q, P);
+    const bool whole = ca == 0;
+    const PolyPart p{c, f, ds, io, da, direct, P, Q, j0 - (long long)(ca * n), m0, m_lo, m_hi, m_lo / Q, m_hi / Q, len, (long long)n,
+                     io.nco ? (const rr::NcoStream*)io.nco->nco_d.p : nullptr, obase, ostride,
+                     rr::tma_input_ok(io.in, io.in_stride, len, S, io.shared), whole, whole && was_ucache_valid && c->allow_ucache};
+    const char* route = nullptr;
+    if (m_hi < m_lo) route = "poly[filter+down]";  // no output fires in this part
+    if constexpr (std::is_same<T, float>::value) {
+        if (!route) RR_TRY(route_fused(p, &route));
+        if (!route) RR_TRY(route_front_poly2(p, &route));
+        if (!route) RR_TRY(route_front_q(p, &route));
+        if (!route) RR_TRY(route_poly2(p, &route));
     }
+    if (!route) RR_TRY(route_poly<T>(p, &route));
+    ds.ztail_stale = true;
+    if (!plan->empty() && plan->back() != '+' && plan->back() != '|' && ca > 0) *plan += "|";
+    *plan += route;
     return RR_OK;
 }
 

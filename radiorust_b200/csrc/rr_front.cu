@@ -29,12 +29,12 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 
-#include <mutex>
 #include <type_traits>
 
 #include "rr_kernels.h"
 #include "rr_poly.cuh"
 #include "rr_pk.cuh"
+#include "rr_tma.cuh"
 
 namespace rr {
 
@@ -384,60 +384,39 @@ __global__ void __launch_bounds__(FR_WARPS * 32, 4) k_front(const __grid_constan
     }
 }
 
-using EncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                              const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeFn front_encode_fn() {
-    static EncodeFn fn = nullptr;
-    static std::once_flag once;
-    std::call_once(once, [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeFn>(p);
-    });
-    return fn;
-}
-
 }  // namespace
 
 bool front_supported(int rank_pad, long long P) {
     // even P (TMA rows are 16-byte multiples; the tile pitch is padded to an odd number of 16-byte units); one TMA
     // box per tile
-    return (rank_pad == 10 || rank_pad == 16) && P >= 2 && P <= 254 && (P % 2) == 0 && front_encode_fn() != nullptr;
+    return (rank_pad == 10 || rank_pad == 16) && P >= 2 && P <= 254 && (P % 2) == 0 && tma_encode_fn() != nullptr;
 }
 
-cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a0, bool shared, cudaStream_t st) {
-    EncodeFn enc = front_encode_fn();
-    if (!enc || (rank_pad != 10 && rank_pad != 16)) return cudaErrorNotSupported;
+cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a0, bool shared, int sm_count, cudaStream_t st) {
+    if (!tma_encode_fn() || (rank_pad != 10 && rank_pad != 16)) return cudaErrorNotSupported;
     FrontArgs a = a0;
     const int tiles = (a.n_rows + FR_ROWS - 1) / FR_ROWS;
     // long-lived warps amortise the per-CTA tables: as few CTAs per stream as keep ~4 CTAs per SM in the
     // grid, the tiles spread evenly over their warps
     int ctas = (tiles + FR_WARPS * 64 - 1) / (FR_WARPS * 64);
-    while ((long long)n_streams * ctas < 592 && ctas * FR_WARPS < tiles) ++ctas;
+    while ((long long)n_streams * ctas < 4LL * sm_count && ctas * FR_WARPS < tiles) ++ctas;
     a.tiles_per_warp = (tiles + ctas * FR_WARPS - 1) / (ctas * FR_WARPS);
-    // the stream as overlapping rows of P samples: element (c0, i, s) = in[s*in_stride + c0 + i*P].  shared: one row
-    // that every stream reads, mapped once (a zero stride cannot be encoded)
-    if (shared != (n_streams > 1 && a.in_stride == 0)) return cudaErrorInvalidValue;
+    // the stream as overlapping rows of P samples: element (c0, i, s) = in[s*in_stride + c0 + i*P]
+    TmaRows rows;
+    if (!tma_input_rows(a.in, a.in_stride, a.len, n_streams, shared, &rows)) return cudaErrorInvalidValue;
     CUtensorMap tm;
-    const cuuint64_t dims[3] = {(cuuint64_t)a.len, (cuuint64_t)FR_ROWS, (cuuint64_t)(shared ? 1 : n_streams)};
-    const cuuint64_t sstride = n_streams > 1 && !shared ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
-    const cuuint64_t strides[2] = {(cuuint64_t)a.P * 8, sstride};
+    const cuuint64_t dims[3] = {(cuuint64_t)a.len, (cuuint64_t)FR_ROWS, rows.count};
+    const cuuint64_t strides[2] = {(cuuint64_t)a.P * 8, rows.stride};
     const int pitch = a.P + ((a.P & 3) == 0 ? 2 : 0);
     const cuuint32_t box[3] = {(cuuint32_t)pitch, (cuuint32_t)FR_ROWS, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    const CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, const_cast<void*>(a.in), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
+    if (!tma_encode(&tm, 3, a.in, dims, strides, box)) return cudaErrorInvalidValue;
     // the history as the same kind of map: element (c0, i, s) = hist2[s*2n + c0 + i*P]
     CUtensorMap tmh = tm;
     a.has_hist_map = 0;
     if (a.hist2 && a.n > 0 && ((uintptr_t)a.hist2 % 16) == 0 && 2 * a.n >= (long long)FR_ROWS * a.P + pitch) {
         const cuuint64_t hdims[3] = {(cuuint64_t)(2 * a.n), (cuuint64_t)FR_ROWS, (cuuint64_t)n_streams};
         const cuuint64_t hstrides[2] = {(cuuint64_t)a.P * 8, (cuuint64_t)(2 * a.n) * 8};
-        if (enc(&tmh, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, const_cast<void*>(a.hist2), hdims, hstrides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS)
-            a.has_hist_map = 1;
+        if (tma_encode(&tmh, 3, a.hist2, hdims, hstrides, box)) a.has_hist_map = 1;
     }
     const int tile_stride = (FR_ROWS * pitch * 8 + 127) / 128 * 128;
     const size_t smem = (size_t)FR_WARPS * FR_STAGES * tile_stride + (size_t)(a.P / 2 + 1) * front_coef_pitch(rank_pad) + (size_t)a.P * 8 + FR_WARPS * FR_STAGES * 8 + 16;

@@ -29,11 +29,11 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
-#include <mutex>
 
 #include "rr_kernels.h"
 #include "rr_poly.cuh"
 #include "rr_pk.cuh"
+#include "rr_tma.cuh"
 
 namespace rr {
 
@@ -56,13 +56,6 @@ constexpr int kFusedSlots = 6;
 constexpr int kFusedSlotFloats = 2560;  // P <= 256
 __constant__ float4 c_fcoef[kFusedSlots * kFusedSlotFloats / 4];
 
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mb_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mb_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void mb_arrive(uint32_t bar) {
     asm volatile("mbarrier.arrive.release.cta.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
@@ -95,24 +88,6 @@ __device__ __forceinline__ void mb_wait_long(uint32_t bar, uint32_t parity) {
         "r"(parity), "r"(20000u)
         : "memory");
 }
-__device__ __forceinline__ pc f_lds(uint32_t addr) {
-    pc r;
-    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(r.x), "=f"(r.y) : "r"(addr));
-    return r;
-}
-__device__ __forceinline__ void f_lds2(uint32_t addr, pc& a, pc& b) {
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(a.x), "=f"(a.y), "=f"(b.x), "=f"(b.y) : "r"(addr));
-}
-__device__ __forceinline__ void f_sts(uint32_t addr, pc a) {
-    asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(addr), "f"(a.x), "f"(a.y) : "memory");
-}
-__device__ __forceinline__ void f_sts2(uint32_t addr, pc a, pc b) {
-    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y) : "memory");
-}
-__device__ __forceinline__ void f_ldg2(const float4* p, pc& a, pc& b) {
-    asm volatile("ld.global.nc.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(a.x), "=f"(a.y), "=f"(b.x), "=f"(b.y) : "l"(p));
-}
-
 // exp(j * sign * 2*pi * (numer*d mod denom) / denom), the phase advance over d samples: rr_poly.cuh's nco_rotation (same
 // integer phase, same double-precision evaluation) without its 64-bit divisions; inv_m = 1 / denom
 __device__ __forceinline__ pc f_rotation(uint32_t d, uint32_t numer_abs, uint32_t denom, double inv_m, int sign) {
@@ -120,20 +95,6 @@ __device__ __forceinline__ pc f_rotation(uint32_t d, uint32_t numer_abs, uint32_
     double s, c;
     sincospi(2.0 * (double)r / (double)denom, &s, &c);
     return pc((float)c, (float)(sign < 0 ? -s : s));
-}
-
-// pass 1 of the 512-point transform of this thread's 32 inputs (rows t + 16*i1), as in rr_poly2.cu
-__device__ __forceinline__ void f_pass1_store(pc (&v)[32], uint32_t tw_row, uint32_t xch_wr) {
-    pdft_regs<32, +1>(v);
-    pc w[3][2];
-    f_lds2(tw_row, w[0][0], w[0][1]);
-    f_lds2(tw_row + 16, w[1][0], w[1][1]);
-#pragma unroll
-    for (int m = 0; m < 16; ++m) {
-        if (m + 2 < 16) f_lds2(tw_row + (m + 2) * 16, w[(m + 2) % 3][0], w[(m + 2) % 3][1]);
-        f_sts(xch_wr + (2 * m) * PITCH, pcmul(v[2 * m], w[m % 3][0]));
-        f_sts(xch_wr + (2 * m + 1) * PITCH, pcmul(v[2 * m + 1], w[m % 3][1]));
-    }
 }
 
 // RR_FUSED_PROF: per-phase cycle counters of front-end warp 0 / transform warp 0 of every CTA (development builds only)
@@ -210,7 +171,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
     unsigned char* const p_ring = p_ys + (((size_t)NB * YS_STRIDE * 8 + 127) / 128 * 128);
     unsigned char* const p_colph = p_ring + (size_t)FW * D * geo.slot_stride;
     unsigned char* const p_bar = p_colph + (((size_t)FW * P * 8 + 127) / 128 * 128);
-    const uint32_t bar_full = s_u32(p_bar), bar_empty = bar_full + 16, bar_ring = bar_full + 32;
+    const uint32_t bar_full = smem_u32(p_bar), bar_empty = bar_full + 16, bar_ring = bar_full + 32;
     const uint32_t left_cnt = bar_ring + FW * D * 8;  // per stage: transform warps that have left it (two 32-bit counters)
 
     // ---- one-time set-up: zero the stages (stale rows must be finite), twiddles, barriers ----------------------
@@ -226,11 +187,11 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
     }
     if (threadIdx.x == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap) : "memory");
-        mb_init(bar_full, FW);
-        mb_init(bar_full + 8, FW);
-        mb_init(bar_empty, T_WARPS);
-        mb_init(bar_empty + 8, T_WARPS);
-        for (int q = 0; q < FW * D; ++q) mb_init(bar_ring + q * 8, 1);
+        mbar_init(bar_full, FW);
+        mbar_init(bar_full + 8, FW);
+        mbar_init(bar_empty, T_WARPS);
+        mbar_init(bar_empty + 8, T_WARPS);
+        for (int q = 0; q < FW * D; ++q) mbar_init(bar_ring + q * 8, 1);
         asm volatile("st.shared.v2.u32 [%0], {%1, %1};" ::"r"(left_cnt), "r"(0u) : "memory");
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -245,7 +206,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
         // overhead competes with 25 steps of ~65 cycles.
         // =====================================================================================================
         const int fw = warp - T_WARPS;
-        const uint32_t ring_s = s_u32(p_ring) + fw * (D * geo.slot_stride);
+        const uint32_t ring_s = smem_u32(p_ring) + fw * (D * geo.slot_stride);
         const uint32_t rbar = bar_ring + fw * (D * 8);
         float2* const colph = reinterpret_cast<float2*>(p_colph) + fw * P;
         const int steps = geo.steps, S0 = geo.S0, hp = geo.hp;
@@ -289,7 +250,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
                 // that starts before the pushed samples (head; patched by hand when the tile is consumed)
                 const int sh = pos0 < 0 ? -1 : F_ROWS - rows_ok;
                 if (lane == 0) {
-                    mb_expect_tx(rbar + i_slot * 8, (uint32_t)geo.slot_bytes);
+                    mbar_expect_tx(rbar + i_slot * 8, (uint32_t)geo.slot_bytes);
                     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
                                      ring_s + i_slot * geo.slot_stride),
                                  "l"(&tmap), "r"(rbar + i_slot * 8), "r"(pos0 + coff - sh * P), "r"(sh), "r"(SHARED_IN ? 0 : (int)blockIdx.x + so * (int)gridDim.x)
@@ -398,7 +359,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
                         const int col0 = half ? half1_col0 : 0;
                         if (pos0 < 0) {
                             // head tile: row 0 arrived as zeros; fill it from the history (already mixed: un-mix) and the push
-                            float2* dst = reinterpret_cast<float2*>(smem + (slot_s - s_u32(smem)));
+                            float2* dst = reinterpret_cast<float2*>(smem + (slot_s - smem_u32(smem)));
                             const float r0x = __shfl_sync(0xffffffffu, rowph.x, 0), r0y = __shfl_sync(0xffffffffu, rowph.y, 0);
                             for (int cc = lane; cc < hp; cc += 32) {
                                 const int p = col0 + cc;
@@ -421,7 +382,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
                         // plain (non-volatile) shared-memory loads: the compiler pipelines them and the constant-bank loads
                         // over the unrolled steps; the mbarrier wait above (memory clobber) keeps them behind the copy.
                         // slot column of sample column 2*st: 2*st - col0
-                        const float4* __restrict__ xrow = reinterpret_cast<const float4*>(smem + (slot_s - s_u32(smem)) + lane * (hp * 8) - col0 * 8);
+                        const float4* __restrict__ xrow = reinterpret_cast<const float4*>(smem + (slot_s - smem_u32(smem)) + lane * (hp * 8) - col0 * 8);
                         if (to_hist) {
                             // tiles inside the last 2n samples: the Filter's next history = the fully mixed samples
                             // (filters.rs:260 keeps the input chunk); a few tiles per stream, run-time loop
@@ -508,7 +469,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
                         o -= V;
                         ++b;
                     }
-                    const uint32_t dst = s_u32(p_stage) + (uint32_t)((gb0 + b) & 1) * STAGE_BYTES + (Lmax + o) * PITCH;
+                    const uint32_t dst = smem_u32(p_stage) + (uint32_t)((gb0 + b) & 1) * STAGE_BYTES + (Lmax + o) * PITCH;
                     const bool live = row < n_out;
                     const bool keep = live && row >= n_out - Lmax;  // the last Lmax rows of the push are the next push's history rows
 #pragma unroll
@@ -522,7 +483,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
                             y0 = pc(0.f, 0.f);
                             y1 = pc(0.f, 0.f);
                         }
-                        f_sts2(dst + c * 8, y0, y1);
+                        sts_pc2(dst + c * 8, y0, y1);
                         if (keep) keep_o[((row - (n_out - Lmax)) * FRK + c) / 2] = make_float4(y0.x, y0.y, y1.x, y1.y);
                     }
                 }
@@ -553,12 +514,12 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
     const int t = lane >> 1, gg = lane & 1;
     const int g = 2 * warp + gg;  // column of u
     auto sync_t = [&]() { asm volatile("bar.sync 1, %0;" ::"n"(T_THREADS) : "memory"); };
-    const uint32_t stage0 = s_u32(p_stage);
-    const uint32_t tw_row = s_u32(p_tw) + t * (TW_UNITS * 16);
+    const uint32_t stage0 = smem_u32(p_stage);
+    const uint32_t tw_row = smem_u32(p_tw) + t * (TW_UNITS * 16);
     const uint32_t tile_rd = t * PITCH + g * 8;
     const uint32_t xch_wr = 33 * t * PITCH + g * 8;
     const uint32_t xch_rd = t * PITCH + g * 8;
-    const uint32_t keep_s = s_u32(p_keep) + warp * 16;
+    const uint32_t keep_s = smem_u32(p_keep) + warp * 16;
     float2* const ysave = reinterpret_cast<float2*>(p_ys);
     const float4* __restrict__ gtab = reinterpret_cast<const float4*>(a.gtab);
     const int hist_rows_per_lane = (Lmax + 31) / 32;  // <= 12 (Lmax <= 383)
@@ -639,27 +600,27 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
             pc v[32];
             const uint32_t src = stg + tile_rd;
 #pragma unroll
-            for (int m = 0; m < 32; ++m) v[m] = f_lds(src + m * (16 * PITCH));
+            for (int m = 0; m < 32; ++m) v[m] = lds_pc(src + m * (16 * PITCH));
             __syncwarp();  // the strip's rows are consumed by every lane before any lane overwrites them
-            f_pass1_store(v, tw_row, stg + xch_wr);
+            pass1_store<PITCH>(v, tw_row, stg + xch_wr);
         }
         {
             const float4* gp = gtab + tid;
             pc h[16];
 #pragma unroll
-            for (int jj = 0; jj < 8; ++jj) f_ldg2(gp + jj * T_THREADS, h[2 * jj], h[2 * jj + 1]);
+            for (int jj = 0; jj < 8; ++jj) ldg_pc2(gp + jj * T_THREADS, h[2 * jj], h[2 * jj + 1]);
             __syncwarp();
 #pragma unroll
             for (int which = 0; which < 2; ++which) {
                 pc x[16];
 #pragma unroll
-                for (int tr = 0; tr < 16; ++tr) x[tr] = f_lds(stg + xch_rd + (33 * tr + 16 * which) * PITCH);
+                for (int tr = 0; tr < 16; ++tr) x[tr] = lds_pc(stg + xch_rd + (33 * tr + 16 * which) * PITCH);
                 pdft_regs<16, +1>(x);
 #pragma unroll
                 for (int k = 0; k < 16; ++k) acc[which * 16 + k] = pcmul(x[k], h[k]);
                 if (which == 0) {
 #pragma unroll
-                    for (int jj = 0; jj < 8; ++jj) f_ldg2(gp + (8 + jj) * T_THREADS, h[2 * jj], h[2 * jj + 1]);
+                    for (int jj = 0; jj < 8; ++jj) ldg_pc2(gp + (8 + jj) * T_THREADS, h[2 * jj], h[2 * jj + 1]);
                 }
             }
         }
@@ -667,7 +628,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
         // ---- sum the ten partial spectra through the stage, park the block's spectrum ------------------------------
         __syncwarp();
 #pragma unroll
-        for (int j = 0; j < 32; ++j) f_sts(stg + xch_rd + (16 * j) * PITCH, acc[j]);
+        for (int j = 0; j < 32; ++j) sts_pc(stg + xch_rd + (16 * j) * PITCH, acc[j]);
         sync_t();
         if (parked == 0) gb_first = gb;
         {
@@ -678,7 +639,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
 #pragma unroll
                 for (int w = 0; w < T_WARPS; ++w) {
                     pc u0, u1;
-                    f_lds2(src + w * 16, u0, u1);
+                    lds_pc2(src + w * 16, u0, u1);
                     sum = sum + u0;
                     sum = sum + u1;
                 }
@@ -704,7 +665,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
                     const float2 q = ys[t + 16 * i1];
                     v[i1] = active ? pc(q.x, -q.y) : pc(0.f, 0.f);  // conj in, conj out = inverse transform
                 }
-                f_pass1_store(v, tw_row, stg + xch_wr);
+                pass1_store<PITCH>(v, tw_row, stg + xch_wr);
                 __syncwarp();
                 const int gj = gb_first + (active ? job : 0);
                 const int so_j = gj / B, b_j = gj - so_j * B;
@@ -715,7 +676,7 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
                 for (int which = 0; which < 2; ++which) {
                     pc x[16];
 #pragma unroll
-                    for (int tr = 0; tr < 16; ++tr) x[tr] = f_lds(stg + xch_rd + (33 * tr + 16 * which) * PITCH);
+                    for (int tr = 0; tr < 16; ++tr) x[tr] = lds_pc(stg + xch_rd + (33 * tr + 16 * which) * PITCH);
                     pdft_regs<16, +1>(x);
                     if (active) {
 #pragma unroll
@@ -761,20 +722,6 @@ k_fused(const __grid_constant__ CUtensorMap tmap, const FusedArgs a, const int n
 // host side
 // ---------------------------------------------------------------------------
 namespace {
-
-using EncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                              const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeFn fused_encode_fn() {
-    static EncodeFn fn = nullptr;
-    static std::once_flag once;
-    std::call_once(once, [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeFn>(p);
-    });
-    return fn;
-}
 
 template <int FW, int D, int NB> size_t fused_smem(int P, int Lmax) {
     const FusedGeom geo = fused_geom(P);
@@ -828,7 +775,7 @@ cudaError_t launch_cfg(int n_streams, const FusedArgs& a, const CUtensorMap& tm,
 int fused_coef_slots() { return kFusedSlots; }
 
 bool fused_supported(int rank_pad, long long P, int Lmax) {
-    if (rank_pad != FRK || !(P == 50 || P == 40 || P == 20) || fused_encode_fn() == nullptr) return false;  // launch_cfg's instantiations
+    if (rank_pad != FRK || !(P == 50 || P == 40 || P == 20) || tma_encode_fn() == nullptr) return false;  // launch_cfg's instantiations
     if (Lmax < 1 || FK - 1 - Lmax < 128 || Lmax > 383) return false;
     if ((P / 2) * 2 * FRK > kFusedSlotFloats) return false;
     return fused_smem<7, 2, 5>((int)P, Lmax) <= (size_t)227 * 1024;
@@ -838,47 +785,30 @@ cudaError_t fused_upload_coef(int slot, const float* acoef, int P, cudaStream_t 
     if (slot < 0 || slot >= kFusedSlots) return cudaErrorInvalidValue;
     const size_t n = (size_t)(P / 2) * 2 * FRK;
     if (n > (size_t)kFusedSlotFloats) return cudaErrorInvalidValue;
-    return cudaMemcpyToSymbolAsync(c_fcoef, acoef, n * sizeof(float), (size_t)slot * kFusedSlotFloats * sizeof(float), cudaMemcpyHostToDevice, st);
+    return cudaMemcpyToSymbolAsync(c_fcoef, acoef, n * sizeof(float), (size_t)slot * kFusedSlotFloats * sizeof(float), cudaMemcpyDeviceToDevice, st);
 }
 
 cudaError_t launch_fused(int n_streams, const FusedArgs& a0, bool shared, int sm_count, cudaStream_t st) {
-    EncodeFn enc = fused_encode_fn();
-    if (!enc) return cudaErrorNotSupported;
+    if (!tma_encode_fn()) return cudaErrorNotSupported;
     FusedArgs a = a0;
     a.coef_off4 = a.coef_slot * (kFusedSlotFloats / 4);
     // the kept rows of a stream enter the stage by one bulk copy: 16-byte aligned source
     if ((uintptr_t)a.ukeep_in % 16 != 0 || (n_streams > 1 && a.ukeep_in_stride % 2 != 0)) return cudaErrorInvalidValue;
     const FusedGeom geo = fused_geom(a.P);
     // the stream as overlapping rows of P samples: element (c0, i, s) = in[s*in_stride + c0 + i*P]; a box is half a
-    // row wide and F_ROWS rows tall.  shared: one row that every stream reads (a zero stride cannot be encoded; the map
-    // holds the row once and the kernel's shared form addresses it)
-    if (shared != (n_streams > 1 && a.in_stride == 0)) return cudaErrorInvalidValue;
+    // row wide and F_ROWS rows tall
+    TmaRows rows;
+    if (!tma_input_rows(a.in, a.in_stride, a.len, n_streams, shared, &rows)) return cudaErrorInvalidValue;
     CUtensorMap tm;
-    const cuuint64_t dims[3] = {(cuuint64_t)a.len, (cuuint64_t)F_ROWS, (cuuint64_t)(shared ? 1 : n_streams)};
-    const cuuint64_t sstride = n_streams > 1 && !shared ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
-    const cuuint64_t strides[2] = {(cuuint64_t)a.P * 8, sstride};
+    const cuuint64_t dims[3] = {(cuuint64_t)a.len, (cuuint64_t)F_ROWS, rows.count};
+    const cuuint64_t strides[2] = {(cuuint64_t)a.P * 8, rows.stride};
     const cuuint32_t box[3] = {(cuuint32_t)geo.hp, (cuuint32_t)F_ROWS, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    const CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, const_cast<void*>(a.in), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
+    if (!tma_encode(&tm, 3, a.in, dims, strides, box)) return cudaErrorInvalidValue;
     // configuration <front-end warps, ring depth, parked spectra>: seven front-end warps fill the register file next to the five
-    // transform warps (12 warps x 168 registers) and were the fastest measured (RR_FUSED_CFG=1: six front-end warps, eight parked spectra)
-    static int cfg = -1;
-    if (cfg < 0) {
-        cfg = 0;
-        if (const char* e = std::getenv("RR_FUSED_CFG")) cfg = std::atoi(e);
-    }
-    if (shared) {
-        switch (cfg) {
-            case 1: return launch_cfg<6, 2, 8, true>(n_streams, a, tm, sm_count, st);
-            default: return launch_cfg<7, 2, 5, true>(n_streams, a, tm, sm_count, st);
-        }
-    }
-    switch (cfg) {
-        case 1: return launch_cfg<6, 2, 8, false>(n_streams, a, tm, sm_count, st);
-        default: return launch_cfg<7, 2, 5, false>(n_streams, a, tm, sm_count, st);
-    }
+    // transform warps (12 warps x 168 registers) and were the fastest measured (six front-end warps with eight parked spectra
+    // were slower)
+    if (shared) return launch_cfg<7, 2, 5, true>(n_streams, a, tm, sm_count, st);
+    return launch_cfg<7, 2, 5, false>(n_streams, a, tm, sm_count, st);
 }
 
 }  // namespace rr

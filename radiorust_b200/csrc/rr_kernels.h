@@ -210,6 +210,13 @@ template <typename T> int poly_hperm_index(int K, int k);
 template <typename T> size_t poly_smem_bytes(int K, int Q, int G, int nbpc);
 template <typename T> cudaError_t launch_poly(int K, int Q, int G, int n_streams, const PolyArgs<T>& a, cudaStream_t st);
 
+// The pushed samples (len complex f32 per stream, n_streams rows in_stride apart; shared: one row that every stream
+// reads) can be read through a TMA tensor map (rr_tma.cuh): 16-byte aligned base, rows a multiple of 16 bytes apart,
+// fewer than 2^31 samples.  k_poly2, k_front and k_fused on the input need it; their launchers refuse what fails it.
+inline bool tma_input_ok(const void* in, long long in_stride, long long len, int n_streams, bool shared) {
+    return ((uintptr_t)in % 16 == 0) && (n_streams == 1 || shared || in_stride % 2 == 0) && len < (1LL << 31);
+}
+
 // ---- k_poly2 (rr_poly2.cu): the complex-f32, Q == 1 form of the polyphase chain on packed
 // fp32 instructions with TMA-fed tiles.  Same PolyArgs; `gtab` is laid out by poly2_table_index.
 bool poly2_supported(int K, long long P, long long Q);
@@ -218,7 +225,7 @@ size_t poly2_smem_bytes(int G, int nbpc);
 // position (complex elements) of bin k of branch p = r*G + g in the device table
 long long poly2_table_index(int G, int r, int g, int k);
 // shared_in: every stream reads the one row at a.in (a.in_stride == 0, n_streams > 1); a zero stride without it is refused
-cudaError_t launch_poly2(int G, int n_streams, const PolyArgs<float>& a, bool shared_in, cudaStream_t st);
+cudaError_t launch_poly2(int G, int n_streams, const PolyArgs<float>& a, bool shared_in, int sm_count, cudaStream_t st);
 
 // ---- k_front (rr_front.cu): rank-reduced front end u_c[i] = sum_p a_c[p] * x'[i*P + p] (f32, Q == 1).
 // k_poly2 then runs on u as a stream of `rank_pad` branches.
@@ -250,7 +257,7 @@ struct FrontArgs {
     int kept_rows;
 };
 bool front_supported(int rank_pad, long long P);
-cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a, bool shared_in, cudaStream_t st);  // shared_in: as launch_poly2
+cudaError_t launch_front(int rank_pad, int n_streams, const FrontArgs& a, bool shared_in, int sm_count, cudaStream_t st);  // shared_in: as launch_poly2
 // k_front_wide (rr_front_wide.cu): the same front end for any P (odd, thousands), 16 or 32 columns; `acoef` is
 // [P][rank_pad]; kept rows are not taken
 bool front_wide_supported(int rank_pad, long long P);
@@ -287,7 +294,7 @@ struct FusedArgs {
 };
 bool fused_supported(int rank_pad, long long P, int Lmax);
 int fused_coef_slots();
-cudaError_t fused_upload_coef(int slot, const float* acoef, int P, cudaStream_t st);
+cudaError_t fused_upload_coef(int slot, const float* acoef, int P, cudaStream_t st);  // acoef: device memory, as FrontArgs::acoef
 cudaError_t launch_fused(int n_streams, const FusedArgs& a, bool shared_in, int sm_count, cudaStream_t st);  // shared_in: as launch_poly2
 
 // new hist2 = last 2n post-NCO samples of [hist2_in | in]; only entries [j_lo, j_hi) (j_hi < 0: 2n) -- the

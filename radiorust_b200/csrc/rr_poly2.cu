@@ -53,12 +53,11 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
-#include <cstdlib>
-#include <mutex>
 
 #include "rr_kernels.h"
 #include "rr_poly.cuh"
 #include "rr_pk.cuh"
+#include "rr_tma.cuh"
 
 namespace rr {
 
@@ -96,13 +95,6 @@ template <int G> struct P2Cfg {
     static size_t smem_bytes(int nbpc) { return 2 * half_bytes(nbpc); }
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     asm volatile(
         "{\n"
@@ -126,43 +118,6 @@ __device__ __forceinline__ uint32_t atom_add_acqrel_shared(uint32_t addr, uint32
     uint32_t old;
     asm volatile("atom.acq_rel.cta.shared::cta.add.u32 %0, [%1], %2;" : "=r"(old) : "r"(addr), "r"(v) : "memory");
     return old;
-}
-
-__device__ __forceinline__ pc lds_pc(uint32_t addr) {
-    pc r;
-    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(r.x), "=f"(r.y) : "r"(addr));
-    return r;
-}
-__device__ __forceinline__ void lds_pc2(uint32_t addr, pc& a, pc& b) {
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(a.x), "=f"(a.y), "=f"(b.x), "=f"(b.y) : "r"(addr));
-}
-__device__ __forceinline__ void sts_pc(uint32_t addr, pc a) {
-    asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(addr), "f"(a.x), "f"(a.y) : "memory");
-}
-__device__ __forceinline__ void sts_pc2(uint32_t addr, pc a, pc b) {
-    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y) : "memory");
-}
-// read-only table load that stays where it is written (volatile asm keeps its place, so the load is
-// in flight while the warp works on something else)
-__device__ __forceinline__ void ldg_pc2(const float4* p, pc& a, pc& b) {
-    asm volatile("ld.global.nc.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(a.x), "=f"(a.y), "=f"(b.x), "=f"(b.y) : "l"(p));
-}
-
-// pass 1 of the K-point forward transform of this thread's 32 inputs (rows t + 16*i1): radix-32
-// butterfly, twiddles from table row `tw_row` (loaded two steps ahead of their use), element (t, k1)
-// to row 33*t + k1 of the warp's strip
-template <int PITCH>
-__device__ __forceinline__ void pass1_store(pc (&v)[32], uint32_t tw_row, uint32_t xch_wr) {
-    pdft_regs<32, +1>(v);
-    pc w[3][2];
-    lds_pc2(tw_row, w[0][0], w[0][1]);
-    lds_pc2(tw_row + 16, w[1][0], w[1][1]);
-#pragma unroll
-    for (int m = 0; m < 16; ++m) {
-        if (m + 2 < 16) lds_pc2(tw_row + (m + 2) * 16, w[(m + 2) % 3][0], w[(m + 2) % 3][1]);
-        sts_pc(xch_wr + (2 * m) * PITCH, pcmul(v[2 * m], w[m % 3][0]));
-        sts_pc(xch_wr + (2 * m + 1) * PITCH, pcmul(v[2 * m + 1], w[m % 3][1]));
-    }
 }
 
 }  // namespace
@@ -588,42 +543,16 @@ __global__ void __launch_bounds__(2 * P2Cfg<G>::THREADS, 1) k_poly2(const __grid
 // ---------------------------------------------------------------------------
 namespace {
 
-using EncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                              const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeFn encode_fn() {
-    static EncodeFn fn = nullptr;
-    static std::once_flag once;
-    std::call_once(once, [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeFn>(p);
-    });
-    return fn;
-}
-
-template <int G> cudaError_t launch_g(int n_streams, const PolyArgs<float>& a0, const CUtensorMap& tm, bool shared, cudaStream_t st) {
+template <int G>
+cudaError_t launch_g(int n_streams, const PolyArgs<float>& a, const CUtensorMap& tm, bool shared, int sm_count, cudaStream_t st) {
     using C = P2Cfg<G>;
-    PolyArgs<float> a = a0;
-    // EXPERIMENT (RR_P2_ONE_HALF_PER_SM=1): one half per CTA and one CTA per SM -- how fast is a lone half?
-    static const bool exp_one = std::getenv("RR_P2_ONE_HALF_PER_SM") != nullptr;
-    if (exp_one) a.halves = 1;
     const int halves = a.halves == 1 ? 1 : 2;
-    size_t smem = C::half_bytes(a.nbpc) * halves;
-    if (exp_one) smem = std::max(smem, (size_t)120 * 1024);
+    const size_t smem = C::half_bytes(a.nbpc) * halves;
     const int per_cta = a.nbpc * (a.ngrp > 0 ? a.ngrp : 1);
     // one CTA per SM; a half walks through several streams when there are more stream pairs than SMs
-    static int sm_count = 0;
-    if (sm_count == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-        if (sm_count <= 0) sm_count = 1;
-    }
     const unsigned gx = (unsigned)((a.n_blocks + per_cta - 1) / per_cta);
     unsigned gy = (unsigned)((n_streams + halves - 1) / halves);
-    const int slots = sm_count * ((halves == 1 && !exp_one) ? 2 : 1);  // CTAs that can be resident at once
+    const int slots = sm_count * (halves == 1 ? 2 : 1);  // CTAs that can be resident at once
     if ((long long)gx * gy > slots) gy = (unsigned)std::max(1, std::min((int)gy, (slots + (int)gx - 1) / (int)gx));
     const dim3 grid(gx, gy);
     void (*kern)(const CUtensorMap, const PolyArgs<float>, const int);
@@ -659,7 +588,7 @@ int poly2_pick_G(long long P) {
 }
 
 bool poly2_supported(int K, long long P, long long Q) {
-    return K == K2 && Q == 1 && P >= 2 && (P % 2) == 0 && poly2_pick_G(P) != 0 && encode_fn() != nullptr;
+    return K == K2 && Q == 1 && P >= 2 && (P % 2) == 0 && poly2_pick_G(P) != 0 && tma_encode_fn() != nullptr;
 }
 
 size_t poly2_smem_bytes(int G, int nbpc) { return P2Cfg<10>::smem_bytes(nbpc); }
@@ -672,23 +601,18 @@ long long poly2_table_index(int G, int r, int g, int k) {
     return ((((long long)r * 2 + which) * 8 + (k2 >> 1)) * threads + tid) * 2 + (k2 & 1);
 }
 
-cudaError_t launch_poly2(int G, int n_streams, const PolyArgs<float>& a, bool shared, cudaStream_t st) {
-    EncodeFn enc = encode_fn();
-    if (!enc) return cudaErrorNotSupported;
-    // the stream as overlapping rows: element (c0, i_lo, i_hi, s) = in[s*in_stride + c0 + (i_lo + 256*i_hi)*P].
-    // shared: one row that every stream reads, mapped once (a zero stride cannot be encoded).  The low-rate part on u,
-    // streams-as-blocks form included, reads per-stream rows.
-    if (shared != (n_streams > 1 && a.in_stride == 0)) return cudaErrorInvalidValue;
+cudaError_t launch_poly2(int G, int n_streams, const PolyArgs<float>& a, bool shared, int sm_count, cudaStream_t st) {
+    if (!tma_encode_fn()) return cudaErrorNotSupported;
+    // the stream as overlapping rows: element (c0, i_lo, i_hi, s) = in[s*in_stride + c0 + (i_lo + 256*i_hi)*P].  The
+    // low-rate part on u, streams-as-blocks form included, reads per-stream rows.
+    TmaRows rows;
+    if (!tma_input_rows(a.in, a.in_stride, a.len, n_streams, shared, &rows)) return cudaErrorInvalidValue;
     CUtensorMap tm;
-    const cuuint64_t dims[4] = {(cuuint64_t)a.len, (cuuint64_t)ROWS_BOX, (cuuint64_t)(K2 / ROWS_BOX), (cuuint64_t)(shared ? 1 : n_streams)};
-    const cuuint64_t sstride = n_streams > 1 && !shared ? (cuuint64_t)a.in_stride * 8 : (((cuuint64_t)a.len * 8 + 15) / 16) * 16;
-    const cuuint64_t strides[3] = {(cuuint64_t)a.P * 8, (cuuint64_t)a.P * 8 * ROWS_BOX, sstride};
+    const cuuint64_t dims[4] = {(cuuint64_t)a.len, (cuuint64_t)ROWS_BOX, (cuuint64_t)(K2 / ROWS_BOX), rows.count};
+    const cuuint64_t strides[3] = {(cuuint64_t)a.P * 8, (cuuint64_t)a.P * 8 * ROWS_BOX, rows.stride};
     const cuuint32_t box[4] = {(cuuint32_t)G, (cuuint32_t)ROWS_BOX, (cuuint32_t)(K2 / ROWS_BOX), 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    const CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT64, 4, const_cast<void*>(a.in), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
-    if (G == 10) return launch_g<10>(n_streams, a, tm, shared, st);
+    if (!tma_encode(&tm, 4, a.in, dims, strides, box)) return cudaErrorInvalidValue;
+    if (G == 10) return launch_g<10>(n_streams, a, tm, shared, sm_count, st);
     return cudaErrorInvalidValue;
 }
 
