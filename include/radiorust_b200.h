@@ -36,7 +36,7 @@ extern "C" {
 #endif
 
 #define RR_VERSION_MAJOR 0
-#define RR_VERSION_MINOR 5
+#define RR_VERSION_MINOR 6
 
 typedef struct rr_ctx rr_ctx;
 typedef struct rr_chain rr_chain;
@@ -274,6 +274,22 @@ int rr_chain_push_shared(rr_chain* chain, double sample_rate, size_t chunk_len, 
                          void* host_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate);
 int rr_chain_push_shared_device(rr_chain* chain, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in,
                                 void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate);
+/* Every stream is pushed as for rr_chain_push[_device]; the chain's outputs of all streams are added into ONE row:
+ * out[t] = sum over s = 0 .. n_streams-1 of y_s[t], where y_s is what rr_chain_push would have written for stream s
+ * (each y_s[t] already rounded to Flt), accumulated in double in ascending stream order starting from +0.0, then
+ * rounded once to Flt.  *out_count = samples in that row; out_capacity counts samples of the row.  Stream state
+ * (NCO phase, Filter history, resampler rings and partial chunks, ...) stays per stream and advances exactly as for a
+ * per-stream push, so summed and per-stream pushes may be mixed on one chain.  Contract, refusals and failure
+ * handling as for rr_chain_push[_device]; out_count > 0 needs a non-null output.  The transmit side of a
+ * channelizer: n_streams baseband channels, each moved onto its own carrier, summed into the wideband row of one SDR.
+ * A chain ending Upsampler (integer factor 8..256, at most 16 taps per phase) -> FreqShifter interpolates, mixes and
+ * sums in one kernel and forms no per-stream output (plan "synth[upsample+nco+sum]"); any other chain writes the
+ * per-stream outputs into scratch of n_streams * out_count samples on the device and adds them (plan "...|sum").
+ * The host form copies n_streams input rows in and the one row out. */
+int rr_chain_push_summed(rr_chain* chain, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in,
+                         size_t in_stride, void* host_out, size_t out_capacity, size_t* out_count, double* out_sample_rate);
+int rr_chain_push_summed_device(rr_chain* chain, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in,
+                                size_t in_stride, void* dev_out, size_t out_capacity, size_t* out_count, double* out_sample_rate);
 int rr_chain_sync(rr_chain* chain);
 /* Copy `n_samples` samples per stream from one device buffer to another (a buffer of another GPU opened with rr_ipc_open,
  * for example) on the chain's copy stream -- a copy engine, no SM -- behind everything queued on the chain so far: a

@@ -119,6 +119,8 @@ SIGNATURES = {
     "rr_chain_push_device": (_I, [_P, _D, _SZ, _SZ, _P, _SZ, _P, _SZ, _SZ, C.POINTER(_SZ), C.POINTER(_D)]),
     "rr_chain_push_shared": (_I, [_P, _D, _SZ, _SZ, _P, _P, _SZ, _SZ, C.POINTER(_SZ), C.POINTER(_D)]),
     "rr_chain_push_shared_device": (_I, [_P, _D, _SZ, _SZ, _P, _P, _SZ, _SZ, C.POINTER(_SZ), C.POINTER(_D)]),
+    "rr_chain_push_summed": (_I, [_P, _D, _SZ, _SZ, _P, _SZ, _P, _SZ, C.POINTER(_SZ), C.POINTER(_D)]),
+    "rr_chain_push_summed_device": (_I, [_P, _D, _SZ, _SZ, _P, _SZ, _P, _SZ, C.POINTER(_SZ), C.POINTER(_D)]),
     "rr_chain_sync": (_I, [_P]),
     "rr_chain_copy_out_async": (_I, [_P, _P, _SZ, _P, _SZ, _SZ]),
     "rr_chain_set_fast_path": (_I, [_P, _I]),

@@ -57,6 +57,7 @@ def translation_units():
         ("rr_front_wide.o", "rr_front_wide.cu", []),
         ("rr_fused.o", "rr_fused.cu", []),
         ("rr_fourier.o", "rr_fourier.cu", []),
+        ("rr_synth.o", "rr_synth.cu", []),
     ]
     for t, tn in (("float", "f32"), ("double", "f64")):
         for k in (256, 512, 1024):

@@ -442,6 +442,56 @@ class Chain:
         )
         return cnt.value, rate.value
 
+    def push_summed(self, sample_rate: float, x: np.ndarray, chunk_len: int, out: Optional[np.ndarray] = None):
+        """Push ``x`` ([n_streams, n_chunks*chunk_len] or 1-D for one stream) from HOST memory and get back ONE row, the
+        sum over streams of what :meth:`push` would return (``rr_chain_push_summed``): a transmit channelizer's
+        wideband output.  Returns ``(y, out_rate)`` with ``y`` of shape ``[out_count]``."""
+        x = np.asarray(x)
+        if x.ndim == 1:
+            x = x[None, :]
+        assert x.shape[0] == self.n_streams, "one row per stream"
+        assert x.dtype == self.cdtype and x.strides[1] == x.itemsize
+        total = x.shape[1]
+        assert total % chunk_len == 0
+        n_chunks = total // chunk_len if chunk_len else 0
+        cap = self.max_output(sample_rate, chunk_len, n_chunks)
+        if out is None:
+            out = np.empty((max(cap, 1),), dtype=self.cdtype)
+        assert out.ndim == 1 and out.dtype == self.cdtype and out.strides[0] == out.itemsize
+        cnt = C.c_size_t()
+        rate = C.c_double()
+        check(
+            self._lib.rr_chain_push_summed(
+                self._h, float(sample_rate), chunk_len, n_chunks, x.ctypes.data, x.strides[0] // x.itemsize,
+                out.ctypes.data, out.shape[0], C.byref(cnt), C.byref(rate),
+            )
+        )
+        self.sync()
+        return out[: cnt.value], rate.value
+
+    def push_summed_device(self, sample_rate, chunk_len, n_chunks, dev_in: int, in_stride: int, dev_out: int, out_capacity: int):
+        """``rr_chain_push_summed_device`` (raw device pointers): the sum over streams into the one row at ``dev_out``;
+        returns ``(out_count, out_rate)``; asynchronous."""
+        cnt = C.c_size_t()
+        rate = C.c_double()
+        check(
+            self._lib.rr_chain_push_summed_device(
+                self._h, float(sample_rate), chunk_len, n_chunks, dev_in, in_stride, dev_out, out_capacity, C.byref(cnt), C.byref(rate),
+            )
+        )
+        return cnt.value, rate.value
+
+    def push_summed_host_async(self, sample_rate, chunk_len, n_chunks, host_in: int, in_stride: int, host_out: int, out_capacity: int):
+        """``rr_chain_push_summed`` with raw (pinned) host pointers; asynchronous until :meth:`sync`."""
+        cnt = C.c_size_t()
+        rate = C.c_double()
+        check(
+            self._lib.rr_chain_push_summed(
+                self._h, float(sample_rate), chunk_len, n_chunks, host_in, in_stride, host_out, out_capacity, C.byref(cnt), C.byref(rate),
+            )
+        )
+        return cnt.value, rate.value
+
     def copy_out_async(self, dst_dev: int, dst_stride: int, src_dev: int, src_stride: int, n_samples: int):
         """``rr_chain_copy_out_async``: copy-engine copy of a push's outputs (raw device pointers), behind the queued work."""
         check(self._lib.rr_chain_copy_out_async(self._h, dst_dev, dst_stride, src_dev, src_stride, n_samples))

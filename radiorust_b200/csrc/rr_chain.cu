@@ -285,6 +285,7 @@ struct rr_chain {
     // kernels and D2H copy are still in flight (PCIe is full duplex; the chain edges are the only PCIe traffic)
     cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr;
     DevBuf stage_in[2], stage_out[2];
+    DevBuf sum_rows;  // summed pushes off the k_synth route: the per-stream outputs, added into the caller's row
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_comp[2] = {nullptr, nullptr}, ev_d2h[2] = {nullptr, nullptr};
     cudaEvent_t ev_copy = nullptr;
     int slot = 0;
@@ -558,8 +559,9 @@ int stage_supported(const rr_chain* c, const rr_stage_desc& d, const Shape& in) 
     return RR_OK;
 }
 
-// output shape of a push without touching any state (capacity check, rr_chain_max_output)
-int dry_shape(const rr_chain* c, const Shape& in, Shape* out) {
+// output shape of a push without touching any state (capacity check, rr_chain_max_output); states (optional): every
+// stage's host state as the push would leave it
+int dry_shape(const rr_chain* c, const Shape& in, Shape* out, std::vector<StageHost>* states = nullptr) {
     std::vector<StageHost> hs;
     hs.reserve(c->st.size());
     for (const auto& s : c->st) hs.push_back(s.h);
@@ -575,6 +577,7 @@ int dry_shape(const rr_chain* c, const Shape& in, Shape* out) {
         sh = a.out;
     }
     *out = sh;
+    if (states) *states = std::move(hs);
     return RR_OK;
 }
 
@@ -1749,11 +1752,23 @@ int run_filter_down(rr_chain* c, Stage& f, Stage& ds, const FilterIo& io, const 
     return RR_OK;
 }
 
+// The summed push's fused route (k_synth): the chain ends Upsampler -> FreqShifter, the Upsampler takes
+// k_upsample_phase's integer-factor form in this push (`up`: its state after the push's dry run), and the push emits.
+bool synth_route(const rr_chain* c, const std::vector<StageHost>& hs, const Shape& out) {
+    const int ns = (int)c->st.size();
+    if (ns < 2 || c->st[ns - 2].d.kind != RR_STAGE_UPSAMPLE || c->st[ns - 1].d.kind != RR_STAGE_FREQSHIFT || out.len() == 0) return false;
+    const StageHost& up = hs[ns - 2];
+    return up.r_valid && !up.r_indexed && rr::upsample_phase_supported(rr::RateState{up.P, up.Q, 0, 0}, up.r_L, (long long)out.len());
+}
+
 // shared: every stream reads the row at dev_in (in_stride is 0).  The stride travels with the input view, so every
 // stage that reads the push's input sees it; the TMA launchers take their shared-row form on a zero stride.
+// summed: dev_out is ONE row (out_stride unused) that receives the sum over streams of the per-stream outputs
+// (rr_chain_push_summed).  Off the k_synth route the stages write the per-stream outputs into c->sum_rows exactly as a
+// per-stream push writes the caller's buffer, and k_stream_sum adds them into the row.
 template <typename T>
 int run_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride, bool shared,
-             void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_rate) {
+             bool summed, void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_rate) {
     const int S = c->S;
     const int ns = (int)c->st.size();
     cudaStream_t st = c->stream;
@@ -1765,11 +1780,21 @@ int run_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks,
     else if (chunk_len * n_chunks > in_stride && S > 1) return fail(RR_ERR_INVALID, "in_stride smaller than the pushed samples");
 
     // ---- dry run: output shape + capacity before anything is touched -------
+    bool synth = false;
+    void* const row_out = dev_out;  // summed: the caller's row
     {
         Shape sh;
-        RR_TRY(dry_shape(c, in, &sh));
+        std::vector<StageHost> hs;
+        RR_TRY(dry_shape(c, in, &sh, &hs));
         if (sh.len() > out_capacity) return fail(RR_ERR_CAPACITY, "output buffer too small for this push");
-        if (sh.len() > out_stride && S > 1) return fail(RR_ERR_INVALID, "out_stride smaller than the produced samples");
+        if (!summed && sh.len() > out_stride && S > 1) return fail(RR_ERR_INVALID, "out_stride smaller than the produced samples");
+        if (summed && sh.len() > 0 && !dev_out) return fail(RR_ERR_INVALID, "rr_chain_push_summed_device: dev_out is null");
+        if (summed) synth = synth_route(c, hs, sh);
+        if (summed && !synth && sh.len() > 0) {
+            RR_TRY(c->sum_rows.ensure((size_t)S * sh.len() * c->esz));
+            dev_out = c->sum_rows.p;
+            out_stride = sh.len();
+        }
     }
 
     c->push_mutated = true;
@@ -2040,6 +2065,48 @@ int run_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks,
             case RR_STAGE_UPSAMPLE: {
                 const bool down = s.d.kind == RR_STAGE_DOWNSAMPLE;
                 if (a.redesign) RR_TRY(resampler_redesign<T>(c, s, cur.sh.rate));
+                if (synth && i == ns - 2) {
+                    // Upsampler -> FreqShifter -> sum in k_synth: the Upsampler's state (carried sums, the pending part
+                    // behind the last whole chunk) and the NCO advance exactly as in a per-stream push.  The staging
+                    // buffers hold only the pending parts, less than one output chunk per stream.
+                    const long long emit = (long long)a.out.len();
+                    RR_TRY(obuf_reserve<T>(c, s, std::max<size_t>(a.pending_before, a.pending_before + a.n_new - (size_t)emit), a.pending_before));
+                    Stage& fs = c->st[i + 1];
+                    StageAct fa;
+                    RR_TRY(advance_stage(fs.d, fs.h, a.out, &fa));
+                    RR_TRY(nco_refresh<T>(c, fs, a.out.rate, fa.nco_recalc));
+                    rr::SynthArgs sa{};
+                    sa.in = cur.p;
+                    sa.in_stride = cur.stride;
+                    sa.len = len;
+                    sa.acc_in = s.tail[s.tail_cur].p;
+                    sa.acc_out = s.tail[s.tail_cur ^ 1].p;
+                    sa.ir = s.ir.p;
+                    sa.L = s.h.r_L;
+                    sa.Q = (int)s.h.Q;
+                    sa.j0 = a.j0;
+                    sa.m0 = a.m0;
+                    sa.n_new = (long long)a.n_new;
+                    sa.pend = s.obuf[s.obuf_cur].p;
+                    sa.pending = (long long)a.pending_before;
+                    sa.rem = s.obuf[s.obuf_cur ^ 1].p;
+                    sa.obuf_stride = (long long)s.obuf_cap;
+                    sa.split = emit - (long long)a.pending_before;
+                    sa.nco = (const rr::NcoStream*)fs.nco_d.p;
+                    sa.out = dev_out;
+                    sa.emit = emit;
+                    RR_TIMED_LAUNCH(c, "k_synth", 1, rr::launch_synth<T>(sa, S, c->ctx->sm_count, st));
+                    RR_LAUNCH(1, rr::launch_nco_advance((rr::NcoStream*)fs.nco_d.p, S, emit, st));
+                    nco_host_advance(fs, emit);
+                    s.tail_cur ^= 1;
+                    s.obuf_cur ^= 1;  // the remainder now lives in the other staging buffer (emit > 0)
+                    cur.p = dev_out;
+                    cur.stride = 0;
+                    cur.sh = fa.out;
+                    plan += "synth[upsample+nco+sum]";
+                    ++i;  // the FreqShifter stage is done
+                    break;
+                }
                 RR_TRY(obuf_reserve<T>(c, s, a.pending_before + a.n_new, a.pending_before));
                 void* o = (char*)s.obuf[s.obuf_cur].p + a.pending_before * 2 * sizeof(T);
                 rr::RateState rs;
@@ -2090,6 +2157,10 @@ int run_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks,
     // (inactive tail stages, or an empty chain): copy the samples through
     if (cur.sh.len() > 0 && cur.p != dev_out) {
         RR_LAUNCH(1, rr::launch_copy2d<T>(cur.p, cur.stride, dev_out, (long long)out_stride, (long long)cur.sh.len(), S, st));
+    }
+    if (summed && !synth && cur.sh.len() > 0) {
+        RR_TIMED_LAUNCH(c, "k_stream_sum", 1, rr::launch_stream_sum<T>(dev_out, (long long)out_stride, (long long)cur.sh.len(), S, row_out, st));
+        plan += "|sum";
     }
     if (out_count) *out_count = cur.sh.len();
     if (out_rate) *out_rate = cur.sh.rate;
@@ -2604,6 +2675,7 @@ int rr_chain_destroy(rr_chain* c) {
         for (DevBuf* b : bufs) b->release();
         if (s.fused_slot >= 0) fused_slot_release(c->ctx->device, &s);
     }
+    c->sum_rows.release();
     if (c->d2h_stream) cudaStreamSynchronize(c->d2h_stream);
     if (c->h2d_stream) cudaStreamSynchronize(c->h2d_stream);
     for (int k = 0; k < 2; ++k) {
@@ -2729,24 +2801,27 @@ size_t rr_chain_max_output(rr_chain* c, double sample_rate, size_t chunk_len, si
 
 namespace {
 
-// rr_chain_push_device / rr_chain_push_shared_device (shared: one input row for every stream, in_stride ignored)
+// rr_chain_push_device / rr_chain_push_shared_device (shared: one input row for every stream, in_stride ignored) /
+// rr_chain_push_summed_device (summed: one output row, the sum over streams; out_stride ignored)
 int push_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride, bool shared,
-                void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
+                bool summed, void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
     if (!c) return fail(RR_ERR_INVALID, "null chain");
     if (out_count) *out_count = 0;
     if (n_chunks == 0 || chunk_len == 0) return RR_OK;
-    if (!dev_in) return fail(RR_ERR_INVALID, shared ? "rr_chain_push_shared_device: dev_in is null" : "rr_chain_push_device: dev_in is null");
+    if (!dev_in)
+        return fail(RR_ERR_INVALID, shared ? "rr_chain_push_shared_device: dev_in is null"
+                                           : (summed ? "rr_chain_push_summed_device: dev_in is null" : "rr_chain_push_device: dev_in is null"));
     if (chunk_len > (size_t)1 << 30 || n_chunks > (size_t)1 << 30) return fail(RR_ERR_INVALID, "push too large");
     RR_CUDA(cudaSetDevice(c->ctx->device));
     (void)cudaGetLastError();  // a stale error of an unrelated earlier call (another library in the process) is not ours
     c->push_mutated = false;
     int r;
     if (c->dtype == RR_C32)
-        r = run_push<float>(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, shared, dev_out, out_capacity, out_stride, out_count,
-                            out_sample_rate);
+        r = run_push<float>(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, shared, summed, dev_out, out_capacity, out_stride,
+                            out_count, out_sample_rate);
     else
-        r = run_push<double>(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, shared, dev_out, out_capacity, out_stride, out_count,
-                             out_sample_rate);
+        r = run_push<double>(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, shared, summed, dev_out, out_capacity, out_stride,
+                             out_count, out_sample_rate);
     if (r != RR_OK && c->push_mutated) {
         // A failure behind the dry run (allocation, CUDA error) left some stages advanced and others not.  The stream
         // cannot be continued consistently: every block restarts as after rr_chain_create (parameters kept; Filters
@@ -2760,13 +2835,15 @@ int push_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chun
     return r;
 }
 
-// rr_chain_push / rr_chain_push_shared (shared: one input row of len samples is staged and read by every stream)
+// rr_chain_push / rr_chain_push_shared (shared: one input row of len samples is staged and read by every stream) /
+// rr_chain_push_summed (summed: one output row of max_out samples is staged and copied back)
 int push_host(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in, size_t in_stride, bool shared,
-              void* host_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
+              bool summed, void* host_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
     if (!c) return fail(RR_ERR_INVALID, "null chain");
     if (out_count) *out_count = 0;
     if (n_chunks == 0 || chunk_len == 0) return RR_OK;
-    if (!host_in) return fail(RR_ERR_INVALID, shared ? "rr_chain_push_shared: host_in is null" : "rr_chain_push: host_in is null");
+    if (!host_in)
+        return fail(RR_ERR_INVALID, shared ? "rr_chain_push_shared: host_in is null" : (summed ? "rr_chain_push_summed: host_in is null" : "rr_chain_push: host_in is null"));
     RR_CUDA(cudaSetDevice(c->ctx->device));
     const size_t len = chunk_len * n_chunks;
     const size_t S = (size_t)c->S;
@@ -2779,8 +2856,9 @@ int push_host(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks
     RR_TRY(dry_shape(c, sh_in, &sh_out));
     const size_t max_out = sh_out.len();
     if (max_out > out_capacity) return fail(RR_ERR_CAPACITY, "output buffer too small for this push");
-    if (max_out > 0 && !host_out) return fail(RR_ERR_INVALID, "rr_chain_push: host_out is null");
-    if (max_out > out_stride && S > 1) return fail(RR_ERR_INVALID, "out_stride smaller than the produced samples");
+    if (max_out > 0 && !host_out) return fail(RR_ERR_INVALID, summed ? "rr_chain_push_summed: host_out is null" : "rr_chain_push: host_out is null");
+    if (!summed && max_out > out_stride && S > 1) return fail(RR_ERR_INVALID, "out_stride smaller than the produced samples");
+    const size_t out_rows = summed ? 1 : S;
     if (!c->h2d_stream) {
         RR_CUDA(cudaStreamCreateWithFlags(&c->h2d_stream, cudaStreamNonBlocking));
         RR_CUDA(cudaStreamCreateWithFlags(&c->d2h_stream, cudaStreamNonBlocking));
@@ -2795,7 +2873,7 @@ int push_host(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks
     // (a staging buffer that has to grow is freed first: cudaFree waits for the work that still uses it)
     const size_t in_rows = shared ? 1 : S;
     RR_TRY(c->stage_in[b].ensure(in_rows * len * c->esz));
-    RR_TRY(c->stage_out[b].ensure(S * ocap * c->esz));
+    RR_TRY(c->stage_out[b].ensure(out_rows * ocap * c->esz));
     // H2D of this push: behind the kernels of the push before last, which read the same slot
     RR_CUDA(cudaStreamWaitEvent(c->h2d_stream, c->ev_comp[b], 0));
     if (in_rows == 1 || in_stride == len)  // contiguous: one linear copy
@@ -2808,13 +2886,14 @@ int push_host(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks
     RR_CUDA(cudaStreamWaitEvent(c->stream, c->ev_h2d[b], 0));
     RR_CUDA(cudaStreamWaitEvent(c->stream, c->ev_d2h[b], 0));
     size_t produced = 0;
-    RR_TRY(push_device(c, sample_rate, chunk_len, n_chunks, c->stage_in[b].p, len, shared, c->stage_out[b].p, max_out, ocap, &produced,
-                       out_sample_rate));
+    RR_TRY(push_device(c, sample_rate, chunk_len, n_chunks, c->stage_in[b].p, len, shared, summed, c->stage_out[b].p, max_out, ocap,
+                       &produced, out_sample_rate));
     RR_CUDA(cudaEventRecord(c->ev_comp[b], c->stream));
     if (produced > 0) {
         RR_CUDA(cudaStreamWaitEvent(c->d2h_stream, c->ev_comp[b], 0));
-        if ((out_stride == ocap && produced == ocap) || S == 1)
-            RR_CUDA(cudaMemcpyAsync(host_out, c->stage_out[b].p, (S == 1 ? produced : S * ocap) * c->esz, cudaMemcpyDeviceToHost, c->d2h_stream));
+        if ((out_stride == ocap && produced == ocap) || out_rows == 1)
+            RR_CUDA(cudaMemcpyAsync(host_out, c->stage_out[b].p, (out_rows == 1 ? produced : S * ocap) * c->esz, cudaMemcpyDeviceToHost,
+                                    c->d2h_stream));
         else
             RR_CUDA(cudaMemcpy2DAsync(host_out, out_stride * c->esz, c->stage_out[b].p, ocap * c->esz, produced * c->esz, S,
                                       cudaMemcpyDeviceToHost, c->d2h_stream));
@@ -2831,24 +2910,38 @@ extern "C" {
 
 int rr_chain_push_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride,
                          void* dev_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
-    return push_device(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, false, dev_out, out_capacity, out_stride, out_count,
+    return push_device(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, false, false, dev_out, out_capacity, out_stride, out_count,
                        out_sample_rate);
 }
 
 int rr_chain_push_shared_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, void* dev_out,
                                 size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
-    return push_device(c, sample_rate, chunk_len, n_chunks, dev_in, 0, true, dev_out, out_capacity, out_stride, out_count, out_sample_rate);
+    return push_device(c, sample_rate, chunk_len, n_chunks, dev_in, 0, true, false, dev_out, out_capacity, out_stride, out_count,
+                       out_sample_rate);
 }
 
 int rr_chain_push(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in, size_t in_stride,
                   void* host_out, size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
-    return push_host(c, sample_rate, chunk_len, n_chunks, host_in, in_stride, false, host_out, out_capacity, out_stride, out_count,
+    return push_host(c, sample_rate, chunk_len, n_chunks, host_in, in_stride, false, false, host_out, out_capacity, out_stride, out_count,
                      out_sample_rate);
 }
 
 int rr_chain_push_shared(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in, void* host_out,
                          size_t out_capacity, size_t out_stride, size_t* out_count, double* out_sample_rate) {
-    return push_host(c, sample_rate, chunk_len, n_chunks, host_in, 0, true, host_out, out_capacity, out_stride, out_count, out_sample_rate);
+    return push_host(c, sample_rate, chunk_len, n_chunks, host_in, 0, true, false, host_out, out_capacity, out_stride, out_count,
+                     out_sample_rate);
+}
+
+int rr_chain_push_summed(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* host_in, size_t in_stride,
+                         void* host_out, size_t out_capacity, size_t* out_count, double* out_sample_rate) {
+    return push_host(c, sample_rate, chunk_len, n_chunks, host_in, in_stride, false, true, host_out, out_capacity, out_capacity, out_count,
+                     out_sample_rate);
+}
+
+int rr_chain_push_summed_device(rr_chain* c, double sample_rate, size_t chunk_len, size_t n_chunks, const void* dev_in, size_t in_stride,
+                                void* dev_out, size_t out_capacity, size_t* out_count, double* out_sample_rate) {
+    return push_device(c, sample_rate, chunk_len, n_chunks, dev_in, in_stride, false, true, dev_out, out_capacity, out_capacity, out_count,
+                       out_sample_rate);
 }
 
 // Device-to-device copy of `n_samples` samples per stream on the chain's copy stream (copy engine, no SM), ordered

@@ -84,6 +84,36 @@ cudaError_t launch_upsample(const void* in, long long in_stride, long long len, 
                             const T* ir, int L, RateState rate, long long n_out, void* out, long long out_stride,
                             int n_streams, cudaStream_t st, void* out2 = nullptr, long long out2_stride = 0, long long out_split = 0);
 template <typename T> bool upsample_tiled_supported(RateState rate, int L);
+// the integer factors that launch_upsample runs one output phase per thread (k_upsample_phase), taps in registers
+inline bool upsample_phase_supported(RateState rate, int L, long long n_out) {
+    return rate.P == 1 && rate.Q >= 8 && rate.Q <= 256 && L >= 1 && (L + rate.Q - 1) / rate.Q <= 16 && n_out + L < (1LL << 40);
+}
+
+// ---- summed-output pushes (rr_synth.cu) ---------------------------------------
+// k_synth: the chain's last two stages Upsampler (upsample_phase_supported) -> FreqShifter of every stream, added into
+// one row.  Row sample t of the push is the FreqShifter's output t of every stream: the samples pending in the
+// Upsampler's staging buffer for t < pending, its new output o = t - pending behind them.
+struct SynthArgs {
+    const void* in;         // [S][in_stride] complex<T>: the Upsampler's input of this push
+    long long in_stride, len;
+    const void* acc_in;     // [S][L]: partial sums carried into this push
+    void* acc_out;          // [S][L]: outputs o >= n_new, carried into the next push
+    const void* ir;         // [L] T
+    int L, Q;               // taps; in/out = 1/Q
+    long long j0, m0;       // RateState of the push
+    long long n_new;        // new Upsampler outputs per stream
+    const void* pend;       // [S][obuf_stride]: samples pending before the push (pre-NCO)
+    long long pending;
+    void* rem;              // [S][obuf_stride]: outputs o >= split, the Upsampler's next pending part (pre-NCO)
+    long long obuf_stride, split;
+    const NcoStream* nco;   // [S] the FreqShifter's state at the push (read-only)
+    void* out;              // the row: `emit` = pending + split samples
+    long long emit;
+};
+template <typename T> cudaError_t launch_synth(const SynthArgs& a, int n_streams, int sm_count, cudaStream_t st);
+// k_stream_sum: out[t] = sum over s ascending of in[s*in_stride + t], in f64 from +0.0, rounded once to T
+template <typename T>
+cudaError_t launch_stream_sum(const void* in, long long in_stride, long long len, int n_streams, void* out, cudaStream_t st);
 
 // The resamplers with their firing pattern from tables (rates that are not integer valued; the tables replay the
 // reference's f64 `pos` recurrence, resampling.rs:109-111 / :247-266): fire[o] = input sample of this push that output o

@@ -446,7 +446,7 @@ template <typename T>
 cudaError_t launch_upsample(const void* in, long long in_stride, long long len, const void* acc_in, void* acc_out,
                             const T* ir, int L, RateState rate, long long n_out, void* out, long long out_stride,
                             int n_streams, cudaStream_t st, void* out2, long long out2_stride, long long out_split) {
-    if (rate.P == 1 && rate.Q >= 8 && rate.Q <= 256 && L >= 1 && (L + rate.Q - 1) / rate.Q <= 16 && n_out + L < (1LL << 40)) {
+    if (upsample_phase_supported(rate, L, n_out)) {
         // a phase per thread, its taps in registers (rates like 48 kS/s -> 2.4 MS/s: Q = 50, 11 taps per phase)
         const int nt = (int)((L + rate.Q - 1) / rate.Q);
         if (nt <= 4) return launch_upsample_phase<T, 4>(in, in_stride, len, acc_in, acc_out, ir, L, rate, n_out, out, out_stride, n_streams, st, out2, out2_stride, out_split);

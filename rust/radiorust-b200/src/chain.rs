@@ -381,6 +381,50 @@ impl<Flt: GpuFloat> Chain<Flt> {
         Ok(Pushed { count, sample_rate: rate })
     }
 
+    /// A transmit channelizer's push: stream `s` reads `input` at `s * in_stride`, and `output` receives ONE row, the
+    /// sum over streams of what [`Chain::push`] would write (added in f64 in stream order, rounded once).  Only that
+    /// row crosses PCIe back.  Asynchronous when both are pinned: call [`Chain::sync`] before reading `output` or
+    /// modifying `input`.
+    pub fn push_summed(
+        &mut self,
+        sample_rate: f64,
+        chunk_len: usize,
+        n_chunks: usize,
+        input: &[Complex<Flt>],
+        in_stride: usize,
+        output: &mut [Complex<Flt>],
+    ) -> Result<Pushed, Error> {
+        assert!(input.len() >= (self.n_streams - 1) * in_stride + chunk_len * n_chunks, "input slice too short");
+        let (mut count, mut rate) = (0usize, 0f64);
+        check(unsafe {
+            sys::rr_chain_push_summed(
+                self.raw, sample_rate, chunk_len, n_chunks, input.as_ptr() as *const c_void, in_stride, output.as_mut_ptr() as *mut c_void,
+                output.len(), &mut count, &mut rate,
+            )
+        })?;
+        Ok(Pushed { count, sample_rate: rate })
+    }
+
+    /// The same with device pointers: the sum over streams goes to the one row at `dev_out`
+    ///
+    /// # Safety
+    /// `dev_in` must be a device allocation of the chain's device holding `n_streams` rows of `in_stride` complex
+    /// samples, `dev_out` one holding `out_capacity` complex samples.
+    pub unsafe fn push_summed_device(
+        &mut self,
+        sample_rate: f64,
+        chunk_len: usize,
+        n_chunks: usize,
+        dev_in: *const c_void,
+        in_stride: usize,
+        dev_out: *mut c_void,
+        out_capacity: usize,
+    ) -> Result<Pushed, Error> {
+        let (mut count, mut rate) = (0usize, 0f64);
+        check(sys::rr_chain_push_summed_device(self.raw, sample_rate, chunk_len, n_chunks, dev_in, in_stride, dev_out, out_capacity, &mut count, &mut rate))?;
+        Ok(Pushed { count, sample_rate: rate })
+    }
+
     /// Wait for everything enqueued by earlier pushes
     pub fn sync(&mut self) -> Result<(), Error> {
         check(unsafe { sys::rr_chain_sync(self.raw) })
